@@ -18,6 +18,9 @@ run once in the verifier constructors, before any timed region, whatever --warmu
   --impl reference : the reference's CPU path (the oracle restatement, fastest vector backend the host has; the Rust
            crate cannot be built in this image) on all host cores, same metric and config.
   --workload msm --lg K : BASELINE config 4, batched Ristretto MSMs of 2^K terms (whole MSMs per rank).
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the device-resident path returned in its last timed step
+           (per-proof verdict codes, per-batch accept flags) as DIR/<name>.npy in float32.  The inputs depend only on the
+           arguments, so two builds can be compared output for output.
 
 Inputs rotate through a pool of distinct groups larger than L2 (config.l2 says so).
 """
@@ -32,6 +35,8 @@ import time
 
 # one hardware work queue per stream (the default of 8 makes >8 streams share queues and serialise)
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
+# the benchmark may run from a read-only tree and writes nothing into it
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -253,7 +258,10 @@ def main():
     ap.add_argument("--msms", type=int, default=8, help="--workload msm: MSMs per call")
     ap.add_argument("--window", type=int, default=0, help="--workload msm: fix the Pippenger window (bits); 0 = by size")
     ap.add_argument("--check-lg", type=int, default=16, help="--workload msm: compare the first MSM with the CPU oracle up to this size")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's verdicts and batch accept flags as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "rangeproof" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the GPU range-proof workload")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     local_world = int(os.environ.get("LOCAL_WORLD_SIZE", str(world)))
     if args.workload == "msm":
@@ -393,6 +401,11 @@ def main():
     if clk:
         clk.mark_end()
     assert int(h_ok.min()) == 1 and int(d_verdicts.abs().max()) == 0, "a timed batch did not verify"
+    if args.dump_outputs and rank == 0:
+        # every context's last group is the last timed sweep: verdicts[k] and batch_ok[k] are what context k returned for it
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("verdicts", d_verdicts), ("batch_ok", h_ok)):
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.cpu().numpy().astype(np.float32))
     value = world * proofs_per_step * args.steps / (ms_dev * 1e-3)
 
     # ---- e2e: host buffers through the public C-ABI call (H2D + kernels + D2H per group)

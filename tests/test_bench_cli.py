@@ -4,13 +4,16 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def test_bench_help_parses():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0, r.stderr
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in r.stdout
 
 
@@ -34,6 +37,26 @@ def test_msm_workload_reference_arm():
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["unit"] == "terms/s" and d["value"] > 0 and d["config"]["lg_n"] == 10
+
+
+def test_dump_outputs_only_on_the_gpu_rangeproof_path(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "out").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    out = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "1", "--streams", "2", "--group", "2",
+                        "--batch", "64", "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-4000:]
+    d = json.loads([ln for ln in r.stdout.splitlines() if ln.strip()][-1])
+    assert d["steps"] == 3 and d["config"]["proofs_per_step"] == 2 * 2 * 64
+    verdicts, batch_ok = np.load(out / "verdicts.npy"), np.load(out / "batch_ok.npy")
+    assert sorted(p.name for p in out.iterdir()) == ["batch_ok.npy", "verdicts.npy"]
+    assert verdicts.dtype == np.float32 and verdicts.shape == (2, 2 * 64) and not verdicts.any()
+    assert batch_ok.dtype == np.float32 and batch_ok.shape == (2, 2) and (batch_ok == 1).all()
 
 
 def test_both_arms_emit_the_same_config():
