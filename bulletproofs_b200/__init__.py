@@ -39,7 +39,6 @@ SYMBOLS = {
     "bp_msm_batch": (_int, [_vp, _u8p, _u8p, _c.POINTER(_c.c_uint64), _sz, _u8p, _u8p]),
     "bp_msm_batch_device": (_int, [_vp, _vp, _vp, _vp, _sz, _sz, _vp, _vp]),
     "bp_msm_indexed_batch": (_int, [_vp, _vp, _u8p, _c.POINTER(_c.c_uint32), _u8p, _sz, _c.POINTER(_c.c_uint64), _sz, _u8p, _u8p]),
-    "bp_ipp_begin": (_int, [_vp, _vp, _sz, _sz, _u8p, _c.POINTER(_vp)]),
     "bp_ipp_begin_points": (_int, [_vp, _u8p, _u8p, _sz, _u8p, _c.POINTER(_vp)]),
     "bp_ipp_lr": (_int, [_vp, _sz, _u8p, _u8p, _u8p, _u8p]),
     "bp_ipp_fold": (_int, [_vp, _sz, _u8p, _u8p, _u8p, _u8p, _int]),

@@ -5,8 +5,11 @@
 #include <cstdio>
 #include <cstdlib>
 #include <algorithm>
+#include <array>
 #include <cstring>
+#include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 #include "../../include/bpmsm.h"
 #include "kernels.cuh"
@@ -15,20 +18,29 @@ static_assert(BP_TRANSCRIPT_BYTES == 203, "transcript wire size");
 
 namespace {
 
-struct DevBuf {
+// Owned allocation: device memory (cudaMalloc) or pinned host memory (cudaMallocHost), freed by the destructor.  Non-copyable, so a
+// handle or arena can be released only by its owner.  ensure() grows scratch with headroom; alloc() sizes a fixed array exactly.
+template <bool Pinned> struct Buf {
     void *p = nullptr; size_t cap = 0;
-    cudaError_t ensure(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e == cudaSuccess) cap = want;
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    ~Buf() { release(); }
+    cudaError_t ensure(size_t bytes) { return bytes <= cap ? cudaSuccess : alloc(bytes + bytes / 4 + 256); }
+    cudaError_t alloc(size_t bytes) {
+        release();
+        cudaError_t e = Pinned ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
+        if (e == cudaSuccess) cap = bytes; else p = nullptr;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    void release() {
+        if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr; cap = 0;
+    }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
+using DevBuf = Buf<false>;
+using HostBuf = Buf<true>;
 
 enum KernelId { KID_DECOMPRESS, KID_COMPRESS, KID_FROM_UNIFORM, KID_MSM_COUNT, KID_MSM_SCAN, KID_MSM_SCATTER, KID_MSM_ACCUMULATE, KID_MSM_REDUCE,
                 KID_MSM_COMBINE, KID_RP_TRANSCRIPT, KID_RP_HEAD, KID_RP_SCALARS, KID_RP_DECOMPRESS, KID_RP_STATIC_REDUCE, KID_IPP_FOLD, KID_SMALL, KID_COUNT };
@@ -41,6 +53,21 @@ struct VerifyState {          // what bp_rangeproof_verify_*begin leaves for *_f
 };
 struct MsmArena { DevBuf counts, starts, cursor, order, sorted, buckets, wsums; };      // scratch of one Pippenger pipeline pass
 struct MsmPlan { int c = 0, W = 0; uint32_t nb = 0, heavy_min = 0; size_t segs = 0, n_buckets = 0, heavy_cap = 0; uint32_t n_msm = 0, T = 0; };
+
+// Everything whose address the verifier's launch graph bakes in (rp_chain's kernel arguments).  Private to the verifier: no other entry
+// point can regrow -- i.e. move -- one of these buffers.  Holds DevBufs only, so signature() walks it as an array and a buffer added
+// here is covered without further bookkeeping.
+struct RpGraphScratch {
+    DevBuf par, contrib, part, scalars, status, decbad, niels, pidx, offsets, results, batch_ok, combined, chal, tabs, raw, pow2_tab;
+    MsmArena ar;
+    uint64_t signature() const {         // FNV-1a over the addresses: a regrown (moved) buffer invalidates the graph
+        const DevBuf *b = reinterpret_cast<const DevBuf *>(this);
+        uint64_t h = 1469598103934665603ULL;
+        for (size_t i = 0; i < sizeof *this / sizeof(DevBuf); i++) { h ^= (uint64_t)(uintptr_t)b[i].p; h *= 1099511628211ULL; }
+        return h;
+    }
+};
+static_assert(std::is_standard_layout<RpGraphScratch>::value && sizeof(RpGraphScratch) % sizeof(DevBuf) == 0, "RpGraphScratch holds DevBufs only");
 
 }  // namespace
 
@@ -55,27 +82,54 @@ struct bp_ctx {
     // MSM scratch
     DevBuf in_scalars, in_points, in_offsets, niels, ok, msm_err, results, outs, flags, ix_pidx;
     MsmArena ar_gen;          // bp_msm*, indexed MSMs, IPP rounds, the verifier's per-proof fallback
-    // range-proof scratch.  Everything the verifier's launch graph touches is private to it (rp_*, ar_rp): no other entry point can
-    // regrow -- i.e. move -- a buffer whose address is baked into the captured graph.
-    MsmArena ar_rp;
-    DevBuf rp_niels, rp_results;
-    DevBuf rp_chal, rp_raw, rp_tabs, pow2_tab, rp_proofs, rp_commit, rp_par, rp_contrib, rp_part, rp_scalars, rp_status, rp_decbad, rp_pidx, rp_offsets, rp_verdict, rp_batch_ok, rp_combined;
+    // range-proof scratch.  The inputs and verdicts stay outside rp: the kernels read their addresses from the parameter block
+    // (rp.par), not from graph arguments, so they may move without invalidating the graph.
+    RpGraphScratch rp;
+    DevBuf rp_proofs, rp_commit, rp_verdict;
     DevBuf fb_scalars, fb_pidx, fb_offsets;
-    uint32_t *h_verdict = nullptr; size_t h_verdict_cap = 0;       // pinned
-    uint32_t *h_flag = nullptr;                                      // pinned: combined_ok[BP_MAX_GROUP_BATCHES] | batch_ok[BP_MAX_GROUP_BATCHES]
+    HostBuf h_verdict;                                               // pinned
+    HostBuf h_flag;                                                  // pinned: combined_ok[BP_MAX_GROUP_BATCHES] | batch_ok[BP_MAX_GROUP_BATCHES]
     // pinned staging ring for the per-call parameter block of the verifier: a slot is reused only after the upload queued from it has
     // completed, so back-to-back device-path calls on one context never see each other's parameters
     static const int STAGE_SLOTS = 8;
-    uint8_t *h_stage = nullptr; cudaEvent_t stage_ev[STAGE_SLOTS] = {}; unsigned stage_next = 0;
+    HostBuf h_stage; cudaEvent_t stage_ev[STAGE_SLOTS] = {}; unsigned stage_next = 0;
     VerifyState vs;
-    size_t pidx_key[6] = {0, 0, 0, 0, 0, 0};                        // geometry the cached rp_pidx / rp_offsets were built for
+    size_t pidx_key[6] = {0, 0, 0, 0, 0, 0};                        // geometry the cached rp.pidx / rp.offsets were built for
     // reserved geometry: every arena sized, launch sequence captured as a CUDA graph
-    cudaGraphExec_t graph = nullptr; size_t graph_key[6] = {0, 0, 0, 0, 0, 0}; uint64_t graph_launches = 0, graph_sig = 0;
+    cudaGraphExec_t graph = nullptr; std::array<size_t, 6> graph_key{}; uint64_t graph_launches = 0, graph_sig = 0;
+    ~bp_ctx() {
+        if (graph) cudaGraphExecDestroy(graph);
+        for (cudaEvent_t e : stage_ev) if (e) cudaEventDestroy(e);
+        if (ev_fork) cudaEventDestroy(ev_fork);
+        if (ev_join) cudaEventDestroy(ev_join);
+        if (aux) cudaStreamDestroy(aux);
+        if (own_stream) cudaStreamDestroy(stream);
+    }
 };
 
 struct bp_gens {
     bp_ctx *ctx = nullptr; size_t cap = 0, parties = 0, n_points = 0;
-    ge_niels *d_table = nullptr;       // [B_blinding, B, G[party][i].., H[party][i]..]
+    DevBuf table;                      // n_points entries: [B_blinding, B, G[party][i].., H[party][i]..]
+    ge_niels *d_table() const { return table.as<ge_niels>(); }
+};
+
+struct bp_points {
+    bp_ctx *ctx = nullptr; size_t n = 0;
+    DevBuf pts, idx;                   // n decompressed points; term -> point map of idx_T terms (k_iota_mod over idx_len)
+    size_t idx_T = 0, idx_len = 0;
+};
+
+struct bp_ipp {
+    bp_ctx *ctx = nullptr; uint32_t N = 0;
+    DevBuf pts;                        // [G (N) | H (N) | Q]
+    DevBuf scal, idx, offs;
+};
+
+struct bp_ippx {
+    bp_ctx *ctx = nullptr; uint32_t N = 0, B = 0, n = 0;
+    const ge_niels *d_static = nullptr; DevBuf own_pts;                   // the gens table, or the session's own [G (N) | H (N)]
+    DevBuf d_q;                                                           // B points Q
+    DevBuf a, b, cG, cH, gidx, hidx, scal, pidx, offs, in, outs;
 };
 
 namespace {
@@ -201,8 +255,8 @@ __global__ void k_rp_point_idx(rp_geom g, uint32_t gens_cap, uint32_t gens_parti
     else { uint32_t b = (uint32_t)(i / g.T); t = (uint32_t)(i % g.T); dyn = dyn_base + b * g.count * g.D + (t - g.S); if (t > g.S) t = g.S; }
     uint32_t v;
     if (t < 2) v = t;                                                                       // B_blinding, B
-    else if (t < 2 + g.N) { uint32_t q = t - 2; v = 2 + (q / g.n) * gens_cap + (q % g.n); } // G(n, m) iterator order (generators.rs:207-259)
-    else if (t < g.S) { uint32_t q = t - 2 - g.N; v = 2 + gens_parties * gens_cap + (q / g.n) * gens_cap + (q % g.n); }
+    else if (t < 2 + g.N) { uint32_t q = t - 2; v = gens_slot(0u, q / g.n, q % g.n, gens_cap, gens_parties); }
+    else if (t < g.S) { uint32_t q = t - 2 - g.N; v = gens_slot(1u, q / g.n, q % g.n, gens_cap, gens_parties); }
     else v = BP_POINT_DYNAMIC | dyn;
     out[i] = v;
 }
@@ -237,7 +291,255 @@ __global__ void k_fill_offsets(uint32_t n, uint32_t stride, uint32_t *out) {
     if (i <= n) out[i] = i * stride;
 }
 
-int lg2_exact(size_t v) { int k = 0; while (((size_t)1 << k) < v) k++; return ((size_t)1 << k) == v ? k : -1; }
+// ---------------------------------------------------------------- steps shared by the entry points
+// decompress n points that must all be valid (resident point sets, IPP generators and Q); synchronises
+int decompress_checked(bp_ctx *c, const uint8_t *d_compressed, size_t n, ge_niels *out) {
+    CK(c, c->ok.ensure(n));
+    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(n, 128), 128, 0, c->stream>>>(d_compressed, n, out, c->ok.as<uint8_t>()));
+    std::vector<uint8_t> ok(n);
+    CK(c, cudaMemcpyAsync(ok.data(), c->ok.p, n, cudaMemcpyDeviceToHost, c->stream)); CK(c, cudaStreamSynchronize(c->stream));
+    for (uint8_t v : ok) if (!v) return BP_ERR_INVALID_POINT;
+    return BP_OK;
+}
+// the MSMs of `a` on the generic arena, compressed to d_outs (a.n_msm x 32 B); with d_status, a.d_err turned into status codes
+int msm_to_bytes(bp_ctx *c, const MsmArgs &a, uint8_t *d_outs, uint8_t *d_status) {
+    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    if (rc) return rc;
+    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(a.n_msm, 128), 128, 0, c->stream>>>(c->results.as<ge_ext>(), a.n_msm, d_outs));
+    if (d_status) { LAUNCH(c, KID_SMALL, k_msm_status<<<blocks_for(a.n_msm, 128), 128, 0, c->stream>>>(a.d_err, a.n_msm, d_status)); }
+    return BP_OK;
+}
+// host-buffer forms: the results and status codes the device form left in c->outs / c->flags back to the caller; synchronises
+int msm_copy_out(bp_ctx *c, size_t n_msm, uint8_t *outs, uint8_t *status) {
+    std::vector<uint8_t> st(n_msm);
+    CK(c, cudaMemcpyAsync(outs, c->outs.p, n_msm * 32, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaMemcpyAsync(st.data(), c->flags.p, n_msm, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    if (status) memcpy(status, st.data(), n_msm);
+    return BP_OK;
+}
+
+// ---------------------------------------------------------------- handle construction: a handle reaches the caller only once complete
+int points_from_device(bp_ctx *c, const uint8_t *d_compressed, size_t n, bp_points **out) {
+    std::unique_ptr<bp_points> h(new bp_points()); h->ctx = c; h->n = n;
+    CK(c, h->pts.alloc(n * sizeof(ge_niels)));
+    int rc = decompress_checked(c, d_compressed, n, h->pts.as<ge_niels>());
+    if (rc) return rc;
+    *out = h.release(); return BP_OK;
+}
+// the table is allocated at exactly n_points entries: no headroom on what may be the largest allocation of the process
+int gens_alloc(bp_ctx *c, size_t cap, size_t parties, std::unique_ptr<bp_gens> &g) {
+    if (!c || cap == 0 || parties == 0) return BP_ERR_INVALID_ARGUMENT;
+    CK(c, cudaSetDevice(c->device));
+    g.reset(new bp_gens());
+    g->ctx = c; g->cap = cap; g->parties = parties; g->n_points = 2 + 2 * cap * parties;
+    CK(c, g->table.alloc(g->n_points * sizeof(ge_niels)));
+    return BP_OK;
+}
+int ippx_alloc(bp_ctx *c, size_t N, size_t B, std::unique_ptr<bp_ippx> &s) {
+    if (!c || N == 0 || (N & (N - 1)) || B == 0 || 2 * B * (N + 1) >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;      // power of two (inner_product_proof.rs:67)
+    BUSY_CHECK(c);
+    CK(c, cudaSetDevice(c->device));
+    s.reset(new bp_ippx()); s->ctx = c; s->N = (uint32_t)N; s->B = (uint32_t)B; s->n = (uint32_t)N;
+    size_t BN = B * N;
+    CK(c, s->d_q.alloc(B * sizeof(ge_niels)));
+    for (DevBuf *b : {&s->a, &s->b, &s->cG, &s->cH}) CK(c, b->ensure(BN * sizeof(sc)));
+    CK(c, s->gidx.ensure(N * 4)); CK(c, s->hidx.ensure(N * 4)); CK(c, s->scal.ensure(2 * B * (N + 1) * 32)); CK(c, s->pidx.ensure(2 * B * (N + 1) * 4));
+    CK(c, s->offs.ensure((2 * B + 1) * 4)); CK(c, s->in.ensure(std::max<size_t>(4 * BN * 32, 64 * B))); CK(c, s->outs.ensure(64 * B));
+    return BP_OK;
+}
+int check_scalars_canonical(const uint8_t *s, size_t n) {
+    for (size_t i = 0; i < n; i++) if (sc_geq_l(sc_load(s + 32 * i))) return BP_ERR_NONCANONICAL_SCALAR;
+    return BP_OK;
+}
+// common tail of the two begin forms: Q points, scalar vectors (B x N canonical scalars each; Gf / Hf may be NULL = all ones)
+int ippx_load(bp_ippx *s, const uint8_t *Q, const uint8_t *Gf, const uint8_t *Hf, const uint8_t *a, const uint8_t *b) {
+    bp_ctx *c = s->ctx; cudaStream_t st = c->stream; size_t BN = (size_t)s->B * s->N;
+    for (const uint8_t *v : {a, b}) if (check_scalars_canonical(v, BN)) return BP_ERR_NONCANONICAL_SCALAR;
+    for (const uint8_t *v : {Gf, Hf}) if (v && check_scalars_canonical(v, BN)) return BP_ERR_NONCANONICAL_SCALAR;
+    uint8_t *din = s->in.as<uint8_t>();
+    CK(c, cudaMemcpyAsync(din, a, BN * 32, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(din + BN * 32, b, BN * 32, cudaMemcpyHostToDevice, st));
+    if (Gf) CK(c, cudaMemcpyAsync(din + 2 * BN * 32, Gf, BN * 32, cudaMemcpyHostToDevice, st));
+    if (Hf) CK(c, cudaMemcpyAsync(din + 3 * BN * 32, Hf, BN * 32, cudaMemcpyHostToDevice, st));
+    ippx_geom g{s->N, s->B, s->n};
+    LAUNCH(c, KID_SMALL, k_ippx_init<<<blocks_for(BN, 128), 128, 0, st>>>(g, din, din + BN * 32, Gf ? din + 2 * BN * 32 : nullptr, Hf ? din + 3 * BN * 32 : nullptr,
+                                                                         s->a.as<sc>(), s->b.as<sc>(), s->cG.as<sc>(), s->cH.as<sc>()));
+    CK(c, c->in_points.ensure((size_t)s->B * 32));
+    CK(c, cudaMemcpyAsync(c->in_points.p, Q, (size_t)s->B * 32, cudaMemcpyHostToDevice, st));
+    int rc = decompress_checked(c, c->in_points.as<uint8_t>(), s->B, s->d_q.as<ge_niels>());
+    if (rc) return rc;
+    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)2 * s->B + 1, 256), 256, 0, st>>>(2 * s->B, s->N + 1, s->offs.as<uint32_t>()));
+    return BP_OK;
+}
+
+// ---------------------------------------------------------------- range proofs
+// Parameter checks of verify_multiple_with_rng (mod.rs:358-366) and of from_bytes / verification_scalars
+// that depend only on (proof_len, n, m): one verdict for the whole call, or BP_PROOF_OK to go on.
+uint8_t rp_param_verdict(const bp_gens *gens, size_t proof_len, size_t n, size_t m, rp_geom *g) {
+    if (proof_len % 32 != 0 || proof_len < 7 * 32) return BP_PROOF_FORMAT_ERROR;                 // mod.rs:498-503
+    size_t ne = (proof_len - 7 * 32) / 32;
+    if (ne < 2 || (ne - 2) % 2 != 0 || (ne - 2) / 2 >= 32) return BP_PROOF_FORMAT_ERROR;         // inner_product_proof.rs:375-388
+    size_t k = (ne - 2) / 2;
+    if (!(n == 8 || n == 16 || n == 32 || n == 64)) return BP_PROOF_INVALID_BITSIZE;
+    if (gens->cap < n || gens->parties < m) return BP_PROOF_INVALID_GENERATORS_LENGTH;
+    if (m == 0 || n * m != ((size_t)1 << k) || k > BP_MAX_LG_N) return BP_PROOF_VERIFICATION_ERROR;   // inner_product_proof.rs:204-211
+    g->n = (uint32_t)n; g->m = (uint32_t)m; g->k = (uint32_t)k; g->N = (uint32_t)(n * m);
+    g->D = (uint32_t)(4 + 2 * k + m); g->S = 2 + 2 * g->N; g->proof_len = (uint32_t)proof_len;
+    return BP_PROOF_OK;
+}
+bool rp_set_group(rp_geom *g, size_t count, size_t n_batches) {
+    if (count == 0 || n_batches == 0 || n_batches > BP_MAX_GROUP_BATCHES || count >= (1u << 24)) return false;
+    size_t T = (size_t)g->S + count * g->D;
+    if (T * n_batches >= (1u << 31) || count * n_batches >= (1u << 24)) return false;
+    g->count = (uint32_t)count; g->nbatch = (uint32_t)n_batches; g->T = (uint32_t)T;
+    return true;
+}
+
+// every arena of one launch group (grow-only); after this nothing on the verification path allocates
+int rp_ensure(bp_ctx *c, const rp_geom &g) {
+    size_t total = (size_t)g.count * g.nbatch, TT = (size_t)g.T * g.nbatch;
+    RpGraphScratch &r = c->rp;
+    CK(c, r.par.ensure(sizeof(rp_params)));
+    CK(c, r.contrib.ensure(total * g.S * sizeof(sc))); CK(c, r.scalars.ensure(TT * 32));
+    CK(c, r.part.ensure((size_t)g.nbatch * ((g.count + RP_CHUNK - 1) / RP_CHUNK) * g.S * sizeof(sc)));
+    CK(c, r.status.ensure(total * 4)); CK(c, r.decbad.ensure(total * 4)); CK(c, r.niels.ensure(total * g.D * sizeof(ge_niels)));
+    CK(c, r.pidx.ensure(TT * 4)); CK(c, r.offsets.ensure(((size_t)g.nbatch + 1) * 4)); CK(c, r.results.ensure((size_t)g.nbatch * sizeof(ge_ext)));
+    CK(c, r.batch_ok.ensure((size_t)g.nbatch * 4)); CK(c, r.combined.ensure((size_t)g.nbatch * 4));
+    CK(c, r.chal.ensure(total * sizeof(rp_head))); CK(c, r.tabs.ensure(total * rp_tab_size(g.k, g.m) * sizeof(sc)));
+    CK(c, r.raw.ensure(total * (RP_RAW_U + g.k) * 64));
+    if (c->h_verdict.cap < total * 4) CK(c, c->h_verdict.alloc(total * 4));
+    if (!r.pow2_tab.p) {             // 2^e (e < 64) in Montgomery form, computed once per context with the host build of sc.cuh
+        std::vector<sc> tab(64);
+        for (int e = 0; e < 64; e++) tab[e] = sc_mont_from_u64(1ULL << e);
+        CK(c, r.pow2_tab.ensure(64 * sizeof(sc)));
+        CK(c, cudaMemcpyAsync(r.pow2_tab.p, tab.data(), 64 * sizeof(sc), cudaMemcpyHostToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream));
+    }
+    return msm_ensure(c, r.ar, msm_make_plan((uint32_t)TT, g.nbatch, 0));
+}
+// what a captured graph was built for besides the scratch addresses: the geometry and the table address (a kernel argument of the captured nodes)
+std::array<size_t, 6> rp_graph_key(const bp_gens *gens, const rp_geom &g) { return {g.n, g.m, g.count, g.nbatch, (size_t)(uintptr_t)gens->table.p, g.proof_len}; }
+// term -> point map and MSM offsets of the combined MSMs: depend only on the geometry, rebuilt when it changes
+int rp_build_maps(bp_ctx *c, bp_gens *gens, const rp_geom &g) {
+    size_t key[6] = {g.n, g.m, g.count, g.nbatch, gens->cap, gens->parties};
+    if (memcmp(key, c->pidx_key, sizeof key) == 0) return BP_OK;
+    cudaStream_t s = c->stream;
+    LAUNCH(c, KID_SMALL, k_rp_point_idx<<<blocks_for((size_t)g.T * g.nbatch, 256), 256, 0, s>>>(g, (uint32_t)gens->cap, (uint32_t)gens->parties, g.count, 0, 0, c->rp.pidx.as<uint32_t>()));
+    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)g.nbatch + 1, 256), 256, 0, s>>>(g.nbatch, g.T, c->rp.offsets.as<uint32_t>()));
+    memcpy(c->pidx_key, key, sizeof key);
+    return BP_OK;
+}
+// upload the per-call parameter block through the pinned staging ring, so that the asynchronous upload never reads caller
+// memory after the entry point returns
+int rp_upload_params(bp_ctx *c, const uint8_t *h_transcript, const uint8_t *seed, const uint8_t *d_proofs, const uint8_t *d_commit, uint32_t *d_verdict) {
+    unsigned slot = c->stage_next++ % bp_ctx::STAGE_SLOTS;
+    CK(c, cudaEventSynchronize(c->stage_ev[slot]));                          // the upload that last used this slot is done
+    rp_params *par = reinterpret_cast<rp_params *>(c->h_stage.as<uint8_t>() + 512 * slot);
+    memset(par, 0, sizeof *par);
+    memcpy(par->tstate, h_transcript, BP_TRANSCRIPT_BYTES);
+    if (seed) memcpy(par->seed, seed, 32);
+    else if (getrandom(par->seed, 32, 0) != 32) { c->err = "getrandom failed"; return BP_ERR_CUDA; }
+    par->proofs = d_proofs; par->commitments = d_commit; par->verdict = d_verdict;
+    CK(c, cudaMemcpyAsync(c->rp.par.p, par, sizeof *par, cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaEventRecord(c->stage_ev[slot], c->stream));
+    return BP_OK;
+}
+
+// The launch sequence of one group, launches only (no allocation, no synchronisation: capturable).  Two branches: the
+// decompressions need nothing but the proof bytes and run beside the transcript replay and the head.
+int rp_chain(bp_ctx *c, bp_gens *gens, const rp_geom &g) {
+    cudaStream_t s = c->stream, s2 = c->prof_on ? c->stream : c->aux;
+    const uint32_t total = g.count * g.nbatch;
+    RpGraphScratch &r = c->rp;
+    const rp_params *par = r.par.as<rp_params>();
+    uint8_t *d_scal = r.scalars.as<uint8_t>();
+    if (s2 != s) { CK(c, cudaEventRecord(c->ev_fork, s)); CK(c, cudaStreamWaitEvent(s2, c->ev_fork, 0)); }
+    CK(c, cudaMemsetAsync(r.decbad.p, 0, (size_t)total * 4, s2));
+    const size_t dec_smem = (size_t)(RP_DEC_THREADS / g.D + 2) * (g.proof_len + 32 * g.m);
+    LAUNCH(c, KID_RP_DECOMPRESS, k_rp_decompress<<<blocks_for((size_t)total * g.D, RP_DEC_THREADS), RP_DEC_THREADS, dec_smem, s2>>>(par, g, total, r.niels.as<ge_niels>(), r.decbad.as<uint32_t>()));
+    if (s2 != s) CK(c, cudaEventRecord(c->ev_join, s2));
+    LAUNCH(c, KID_RP_TRANSCRIPT, k_rp_transcript<<<blocks_for(total, RP_TR_THREADS), RP_TR_THREADS, 0, s>>>(par, g, total, r.raw.as<uint8_t>(), r.status.as<uint32_t>()));
+    LAUNCH(c, KID_RP_HEAD, k_rp_head_seq<<<blocks_for(total, 32), 32, 0, s>>>(par, g, r.raw.as<uint8_t>(), total, r.chal.as<rp_head>(), r.tabs.as<sc>(),
+                                                                                  r.pow2_tab.as<sc>(), r.status.as<uint32_t>()));
+    if (s2 != s) CK(c, cudaStreamWaitEvent(s, c->ev_join, 0));
+    const uint32_t nchunks = (g.count + RP_CHUNK - 1) / RP_CHUNK;
+    LAUNCH(c, KID_RP_SCALARS, k_rp_scalars_sum<<<g.nbatch * nchunks, (unsigned)std::min<uint32_t>(128, std::max<uint32_t>(32, g.N)), 0, s>>>(g, r.chal.as<rp_head>(), r.tabs.as<sc>(),
+                                                                                  r.decbad.as<uint32_t>(), r.part.as<sc>(), d_scal));
+    LAUNCH(c, KID_RP_STATIC_REDUCE, k_rp_static_sum<<<dim3(g.S, g.nbatch), 32, 0, s>>>(r.part.as<sc>(), g, d_scal));
+    MsmArgs a{d_scal, r.offsets.as<uint32_t>(), g.nbatch, g.T * g.nbatch, r.pidx.as<uint32_t>(), gens->d_table(), r.niels.as<ge_niels>(), nullptr, 0};
+    int rc = msm_launch(c, r.ar, a, msm_make_plan(a.T, a.n_msm, 0), r.results.as<ge_ext>());
+    if (rc) return rc;
+    LAUNCH(c, KID_SMALL, k_rp_verdict_batch<<<g.nbatch, 256, 0, s>>>(r.status.as<uint32_t>(), r.decbad.as<uint32_t>(), r.results.as<ge_ext>(), g, par,
+                                                                      r.batch_ok.as<uint32_t>(), r.combined.as<uint32_t>()));
+    return BP_OK;
+}
+
+bool rp_graph_matches(const bp_ctx *c, const bp_gens *gens, const rp_geom &g) {
+    return c->graph && rp_graph_key(gens, g) == c->graph_key && c->graph_sig == c->rp.signature();
+}
+// queue everything up to the verdicts; d_proofs / d_commitments are device pointers
+int rp_verify_queue(bp_ctx *c, bp_gens *gens, const rp_geom &g, const uint8_t *d_proofs, const uint8_t *d_commit,
+                    const uint8_t *h_transcript, const uint8_t *seed, uint32_t *d_verdict) {
+    const bool use_graph = !c->prof_on && rp_graph_matches(c, gens, g);
+    if (!use_graph) { int rc = rp_ensure(c, g); if (rc) return rc; }
+    int rc = rp_build_maps(c, gens, g);          // another geometry may have used the context since: the maps follow the key
+    if (rc) return rc;
+    rc = rp_upload_params(c, h_transcript, seed, d_proofs, d_commit, d_verdict);
+    if (rc) return rc;
+    if (use_graph) { CK(c, cudaGraphLaunch(c->graph, c->stream)); c->launches += c->graph_launches; return BP_OK; }
+    return rp_chain(c, gens, g);
+}
+
+// per-proof re-check of the proofs [p0, p0 + count) of a group: count independent MSMs of S + D terms
+int rp_fallback_range(bp_ctx *c, bp_gens *gens, const rp_geom &g, uint32_t p0, uint32_t count, uint32_t *d_verdict) {
+    cudaStream_t s = c->stream;
+    uint32_t row = g.S + g.D; size_t T = (size_t)count * row;
+    if (T >= (1u << 31)) { c->err = "fallback batch too large"; return BP_ERR_INVALID_ARGUMENT; }
+    CK(c, c->fb_scalars.ensure(T * 32)); CK(c, c->fb_pidx.ensure(T * 4)); CK(c, c->fb_offsets.ensure(((size_t)count + 1) * 4));
+    CK(c, c->results.ensure((size_t)count * sizeof(ge_ext)));
+    uint32_t batch = p0 / g.count, q0 = p0 % g.count;
+    const uint8_t *dyn = c->rp.scalars.as<uint8_t>() + ((size_t)batch * g.T + g.S + (size_t)q0 * g.D) * 32;
+    LAUNCH(c, KID_SMALL, k_rp_expand_scalars<<<blocks_for(T, 128), 128, 0, s>>>(c->rp.contrib.as<sc>() + (size_t)p0 * g.S, dyn, g, count, c->fb_scalars.as<uint8_t>()));
+    LAUNCH(c, KID_SMALL, k_rp_point_idx<<<blocks_for(T, 256), 256, 0, s>>>(g, (uint32_t)gens->cap, (uint32_t)gens->parties, count, 1, p0 * g.D, c->fb_pidx.as<uint32_t>()));
+    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)count + 1, 256), 256, 0, s>>>(count, row, c->fb_offsets.as<uint32_t>()));
+    MsmArgs a{c->fb_scalars.as<uint8_t>(), c->fb_offsets.as<uint32_t>(), count, (uint32_t)T, c->fb_pidx.as<uint32_t>(), gens->d_table(), c->rp.niels.as<ge_niels>(), nullptr, 0};
+    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    if (rc) return rc;
+    LAUNCH(c, KID_SMALL, k_rp_verdict_proofs<<<blocks_for(count, 128), 128, 0, s>>>(c->rp.status.as<uint32_t>() + p0, c->rp.decbad.as<uint32_t>() + p0, c->results.as<ge_ext>(), count, d_verdict + p0));
+    return BP_OK;
+}
+// A batch whose combined check failed.  Level 1: one combined MSM per chunk of RP_CHUNK proofs, from the partial sums the main path
+// already holds (one pipeline pass over the batch's ~T terms).  Level 2: the proofs of the failing chunks, each with its own MSM
+// (mod.rs:421-447 per proof).  One bad proof in 1024 costs two small passes instead of 1024 147-term MSMs.
+int rp_verify_fallback(bp_ctx *c, bp_gens *gens, const rp_geom &g, uint32_t batch, uint32_t *d_verdict, bool *contrib_ready) {
+    cudaStream_t s = c->stream;
+    const uint32_t nch = (g.count + RP_CHUNK - 1) / RP_CHUNK, row = g.S + RP_CHUNK * g.D, p0 = batch * g.count;
+    size_t T = (size_t)nch * row;
+    if (T >= (1u << 31)) { c->err = "fallback batch too large"; return BP_ERR_INVALID_ARGUMENT; }
+    CK(c, c->fb_scalars.ensure(T * 32)); CK(c, c->fb_pidx.ensure(T * 4)); CK(c, c->fb_offsets.ensure(((size_t)nch + 1) * 4));
+    CK(c, c->results.ensure((size_t)nch * sizeof(ge_ext))); CK(c, c->flags.ensure((size_t)nch * 4));
+    LAUNCH(c, KID_SMALL, k_rp_chunk_rows<<<blocks_for(T, 128), 128, 0, s>>>(c->rp.part.as<sc>() + (size_t)batch * nch * g.S, c->rp.scalars.as<uint8_t>() + ((size_t)batch * g.T + g.S) * 32, g,
+                                                                              (uint32_t)gens->cap, (uint32_t)gens->parties, p0 * g.D, c->fb_scalars.as<uint8_t>(), c->fb_pidx.as<uint32_t>()));
+    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)nch + 1, 256), 256, 0, s>>>(nch, row, c->fb_offsets.as<uint32_t>()));
+    MsmArgs a{c->fb_scalars.as<uint8_t>(), c->fb_offsets.as<uint32_t>(), nch, (uint32_t)T, c->fb_pidx.as<uint32_t>(), gens->d_table(), c->rp.niels.as<ge_niels>(), nullptr, 0};
+    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    if (rc) return rc;
+    LAUNCH(c, KID_SMALL, k_rp_verdict_chunks<<<blocks_for(g.count, 128), 128, 0, s>>>(c->rp.status.as<uint32_t>() + p0, c->rp.decbad.as<uint32_t>() + p0, c->results.as<ge_ext>(), g.count,
+                                                                                      d_verdict + p0, c->flags.as<uint32_t>()));
+    std::vector<uint32_t> ok(nch);
+    CK(c, cudaMemcpyAsync(ok.data(), c->flags.p, (size_t)nch * 4, cudaMemcpyDeviceToHost, s)); CK(c, cudaStreamSynchronize(s));
+    uint32_t nfail = 0; for (uint32_t v : ok) nfail += v ? 0 : 1;
+    if (nfail == 0) return BP_OK;       // cannot happen when the batch's combination failed, short of a 2^-128 cancellation between chunk weights
+    if (!*contrib_ready) {   // the combined path keeps only sums: the per-proof static-term scalars are produced here, on the reject path (whole group; idempotent)
+        const uint32_t total = g.count * g.nbatch;
+        LAUNCH(c, KID_RP_SCALARS, k_rp_scalars<<<blocks_for((size_t)total * (g.N + g.D), 128), 128, 0, s>>>(g, c->rp.chal.as<rp_head>(), c->rp.tabs.as<sc>(), c->rp.decbad.as<uint32_t>(), total,
+                                                                                                            c->rp.contrib.as<sc>(), c->rp.scalars.as<uint8_t>()));
+        *contrib_ready = true;
+    }
+    if (nfail > 4) return rp_fallback_range(c, gens, g, p0, g.count, d_verdict);      // many bad chunks: one pass over the whole batch
+    for (uint32_t ch = 0; ch < nch; ch++)
+        if (!ok[ch]) { rc = rp_fallback_range(c, gens, g, p0 + ch * RP_CHUNK, std::min<uint32_t>(RP_CHUNK, g.count - ch * RP_CHUNK), d_verdict); if (rc) return rc; }
+    return BP_OK;
+}
 
 }  // namespace
 
@@ -252,18 +554,17 @@ int bp_ctx_create(int device, void *stream, bp_ctx **out) {
     if (cudaSetDevice(device) != cudaSuccess) return BP_ERR_CUDA;
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess || prop.major < 10) return BP_ERR_CUDA;   // sm_100a only
-    bp_ctx *c = new bp_ctx();
+    std::unique_ptr<bp_ctx> c(new bp_ctx());
     c->device = device; c->sm_count = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
     if (stream) { c->stream = (cudaStream_t)stream; c->own_stream = false; }
-    else { if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return BP_ERR_CUDA; } c->own_stream = true; }
-    if (cudaMallocHost((void **)&c->h_flag, 2 * BP_MAX_GROUP_BATCHES * 4) != cudaSuccess) { delete c; return BP_ERR_CUDA; }
-    if (cudaMallocHost((void **)&c->h_stage, 512 * bp_ctx::STAGE_SLOTS) != cudaSuccess) { cudaFreeHost(c->h_flag); delete c; return BP_ERR_CUDA; }
-    for (int i = 0; i < bp_ctx::STAGE_SLOTS; i++) cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming);
-    cudaStreamCreateWithFlags(&c->aux, cudaStreamNonBlocking);
+    else { if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) return BP_ERR_CUDA; c->own_stream = true; }
+    if (c->h_flag.alloc(2 * BP_MAX_GROUP_BATCHES * 4) != cudaSuccess || c->h_stage.alloc(512 * bp_ctx::STAGE_SLOTS) != cudaSuccess) return BP_ERR_CUDA;
+    for (cudaEvent_t &e : c->stage_ev) if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return BP_ERR_CUDA;
+    if (cudaStreamCreateWithFlags(&c->aux, cudaStreamNonBlocking) != cudaSuccess) return BP_ERR_CUDA;
     // k_rp_decompress stages the proofs its block touches in dynamic shared memory: up to 13 proofs of 32*(9+2*20) + 32*m bytes
-    cudaFuncSetAttribute(k_rp_decompress, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming); cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming);
-    *out = c;
+    if (cudaFuncSetAttribute(k_rp_decompress, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess) return BP_ERR_CUDA;
+    if (cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming) != cudaSuccess) return BP_ERR_CUDA;
+    *out = c.release();
     return BP_OK;
 }
 void bp_ctx_destroy(bp_ctx *c) {
@@ -271,19 +572,6 @@ void bp_ctx_destroy(bp_ctx *c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     if (c->aux) cudaStreamSynchronize(c->aux);
-    if (c->graph) cudaGraphExecDestroy(c->graph);
-    DevBuf *bufs[] = {&c->in_scalars, &c->in_points, &c->in_offsets, &c->niels, &c->ok, &c->msm_err, &c->results, &c->outs, &c->flags, &c->ix_pidx, &c->rp_niels, &c->rp_results, &c->rp_chal, &c->rp_raw, &c->rp_tabs, &c->pow2_tab, &c->rp_proofs, &c->rp_commit, &c->rp_par, &c->rp_contrib, &c->rp_part, &c->rp_scalars,
-                      &c->rp_status, &c->rp_decbad, &c->rp_pidx, &c->rp_offsets, &c->rp_verdict, &c->rp_batch_ok, &c->rp_combined, &c->fb_scalars, &c->fb_pidx, &c->fb_offsets};
-    for (DevBuf *b : bufs) b->release();
-    for (MsmArena *ar : {&c->ar_gen, &c->ar_rp}) for (DevBuf *b : {&ar->counts, &ar->starts, &ar->cursor, &ar->order, &ar->sorted, &ar->buckets, &ar->wsums}) b->release();
-    if (c->h_verdict) cudaFreeHost(c->h_verdict);
-    if (c->h_flag) cudaFreeHost(c->h_flag);
-    if (c->h_stage) cudaFreeHost(c->h_stage);
-    for (int i = 0; i < bp_ctx::STAGE_SLOTS; i++) if (c->stage_ev[i]) cudaEventDestroy(c->stage_ev[i]);
-    if (c->ev_fork) cudaEventDestroy(c->ev_fork);
-    if (c->ev_join) cudaEventDestroy(c->ev_join);
-    if (c->aux) cudaStreamDestroy(c->aux);
-    if (c->own_stream) cudaStreamDestroy(c->stream);
     delete c;
 }
 const char *bp_last_error(const bp_ctx *c) { return c ? c->err.c_str() : "null context"; }
@@ -330,11 +618,7 @@ int bp_msm_batch_device(bp_ctx *c, const void *d_scalars, const void *d_points, 
     LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(T, 128), 128, 0, s>>>((const uint8_t *)d_points, T, c->niels.as<ge_niels>(), c->ok.as<uint8_t>()));
     LAUNCH(c, KID_SMALL, k_mark_invalid<<<blocks_for(T, 256), 256, 0, s>>>(c->ok.as<uint8_t>(), (const uint32_t *)d_offsets_u32, M, T, c->msm_err.as<uint32_t>()));
     MsmArgs a{(const uint8_t *)d_scalars, (const uint32_t *)d_offsets_u32, M, T, nullptr, nullptr, c->niels.as<ge_niels>(), c->msm_err.as<uint32_t>(), 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
-    if (rc) return rc;
-    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(M, 128), 128, 0, s>>>(c->results.as<ge_ext>(), M, (uint8_t *)d_outs));
-    if (d_status) { LAUNCH(c, KID_SMALL, k_msm_status<<<blocks_for(M, 128), 128, 0, s>>>(c->msm_err.as<uint32_t>(), M, (uint8_t *)d_status)); }
-    return BP_OK;
+    return msm_to_bytes(c, a, (uint8_t *)d_outs, (uint8_t *)d_status);
 }
 
 int bp_msm_batch(bp_ctx *c, const uint8_t *scalars, const uint8_t *points, const uint64_t *offsets, size_t n_msm, uint8_t *outs, uint8_t *status) {
@@ -357,12 +641,7 @@ int bp_msm_batch(bp_ctx *c, const uint8_t *scalars, const uint8_t *points, const
     CK(c, cudaMemcpyAsync(c->in_offsets.p, off32.data(), (n_msm + 1) * 4, cudaMemcpyHostToDevice, s));
     int rc = bp_msm_batch_device(c, c->in_scalars.p, c->in_points.p, c->in_offsets.p, n_msm, T, c->outs.p, c->flags.p);
     if (rc) return rc;
-    std::vector<uint8_t> st(n_msm);
-    CK(c, cudaMemcpyAsync(outs, c->outs.p, n_msm * 32, cudaMemcpyDeviceToHost, s));
-    CK(c, cudaMemcpyAsync(st.data(), c->flags.p, n_msm, cudaMemcpyDeviceToHost, s));
-    CK(c, cudaStreamSynchronize(s));
-    if (status) memcpy(status, st.data(), n_msm);
-    return BP_OK;
+    return msm_copy_out(c, n_msm, outs, status);
 }
 
 int bp_msm(bp_ctx *c, const uint8_t *scalars, const uint8_t *points, size_t n, uint8_t out[32]) {
@@ -399,26 +678,10 @@ int bp_compress_batch(bp_ctx *c, const uint8_t *xyzt, size_t n, uint8_t *points_
 }
 
 // ---------------------------------------------------------------------------------------------- resident point sets (decompressed once, reused by many MSMs)
-}  // extern "C"
-struct bp_points { bp_ctx *ctx = nullptr; size_t n = 0; ge_niels *d_pts = nullptr; uint32_t *d_idx = nullptr; size_t idx_T = 0, idx_len = 0; };
-extern "C" {
-static int points_from_device(bp_ctx *c, const uint8_t *d_compressed, size_t n, bp_points **out) {
-    bp_points *h = new bp_points(); h->ctx = c; h->n = n;
-    cudaError_t e = cudaMalloc((void **)&h->d_pts, n * sizeof(ge_niels));
-    if (e != cudaSuccess) { c->err = std::string("cudaMalloc(points): ") + cudaGetErrorString(e); delete h; return BP_ERR_CUDA; }
-    int rc = [&]() -> int {
-        CK(c, c->ok.ensure(n));
-        LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(n, 128), 128, 0, c->stream>>>(d_compressed, n, h->d_pts, c->ok.as<uint8_t>()));
-        std::vector<uint8_t> ok(n);
-        CK(c, cudaMemcpyAsync(ok.data(), c->ok.p, n, cudaMemcpyDeviceToHost, c->stream)); CK(c, cudaStreamSynchronize(c->stream));
-        for (uint8_t v : ok) if (!v) return BP_ERR_INVALID_POINT;
-        return BP_OK;
-    }();
-    if (rc) { cudaFree(h->d_pts); delete h; return rc; }
-    *out = h; return BP_OK;
-}
 int bp_points_create(bp_ctx *c, const uint8_t *points, size_t n, bp_points **out) {
-    if (!c || !points || !out || n == 0 || n >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    if (!c || !points || n == 0 || n >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;
     BUSY_CHECK(c);
     CK(c, cudaSetDevice(c->device));
     CK(c, c->in_points.ensure(n * 32));
@@ -426,12 +689,14 @@ int bp_points_create(bp_ctx *c, const uint8_t *points, size_t n, bp_points **out
     return points_from_device(c, c->in_points.as<uint8_t>(), n, out);
 }
 int bp_points_create_device(bp_ctx *c, const void *d_points, size_t n, bp_points **out) {
-    if (!c || !d_points || !out || n == 0 || n >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    if (!c || !d_points || n == 0 || n >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;
     BUSY_CHECK(c);
     CK(c, cudaSetDevice(c->device));
     return points_from_device(c, (const uint8_t *)d_points, n, out);
 }
-void bp_points_destroy(bp_points *h) { if (!h) return; cudaSetDevice(h->ctx->device); cudaStreamSynchronize(h->ctx->stream); cudaFree(h->d_pts); if (h->d_idx) cudaFree(h->d_idx); delete h; }
+void bp_points_destroy(bp_points *h) { if (!h) return; cudaSetDevice(h->ctx->device); cudaStreamSynchronize(h->ctx->stream); delete h; }
 size_t bp_points_count(const bp_points *h) { return h ? h->n : 0; }
 
 // n_msm MSMs of `terms` terms each over the first `terms` points of the set (MSM j uses scalars[j*terms .. (j+1)*terms)); device pointers,
@@ -444,21 +709,16 @@ int bp_msm_points_device(bp_ctx *c, bp_points *h, const void *d_scalars, size_t 
     cudaStream_t s = c->stream;
     if (h->idx_T < T || h->idx_len != terms) {
         CK(c, cudaStreamSynchronize(s));
-        if (h->d_idx) cudaFree(h->d_idx);
-        h->d_idx = nullptr; h->idx_T = 0;
-        CK(c, cudaMalloc((void **)&h->d_idx, (size_t)T * 4));
-        LAUNCH(c, KID_SMALL, k_iota_mod<<<blocks_for(T, 256), 256, 0, s>>>(T, (uint32_t)terms, h->d_idx));
+        h->idx_T = 0;
+        CK(c, h->idx.alloc((size_t)T * 4));
+        LAUNCH(c, KID_SMALL, k_iota_mod<<<blocks_for(T, 256), 256, 0, s>>>(T, (uint32_t)terms, h->idx.as<uint32_t>()));
         h->idx_T = T; h->idx_len = terms;
     }
     CK(c, c->in_offsets.ensure(((size_t)M + 1) * 4)); CK(c, c->msm_err.ensure((size_t)M * 4)); CK(c, c->results.ensure((size_t)M * sizeof(ge_ext)));
     LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)M + 1, 256), 256, 0, s>>>(M, (uint32_t)terms, c->in_offsets.as<uint32_t>()));
     CK(c, cudaMemsetAsync(c->msm_err.p, 0, (size_t)M * 4, s));
-    MsmArgs a{(const uint8_t *)d_scalars, c->in_offsets.as<uint32_t>(), M, T, h->d_idx, h->d_pts, nullptr, c->msm_err.as<uint32_t>(), 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
-    if (rc) return rc;
-    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(M, 128), 128, 0, s>>>(c->results.as<ge_ext>(), M, (uint8_t *)d_outs));
-    if (d_status) { LAUNCH(c, KID_SMALL, k_msm_status<<<blocks_for(M, 128), 128, 0, s>>>(c->msm_err.as<uint32_t>(), M, (uint8_t *)d_status)); }
-    return BP_OK;
+    MsmArgs a{(const uint8_t *)d_scalars, c->in_offsets.as<uint32_t>(), M, T, h->idx.as<uint32_t>(), h->pts.as<ge_niels>(), nullptr, c->msm_err.as<uint32_t>(), 0};
+    return msm_to_bytes(c, a, (uint8_t *)d_outs, (uint8_t *)d_status);
 }
 // host-buffer form (pinned memory recommended): H2D of the scalars, the MSMs, D2H of the 32-byte results; synchronises
 int bp_msm_points(bp_ctx *c, bp_points *h, const uint8_t *scalars, size_t n_msm, size_t terms, uint8_t *outs, uint8_t *status) {
@@ -470,31 +730,26 @@ int bp_msm_points(bp_ctx *c, bp_points *h, const uint8_t *scalars, size_t n_msm,
     CK(c, cudaMemcpyAsync(c->in_scalars.p, scalars, T * 32, cudaMemcpyHostToDevice, c->stream));
     int rc = bp_msm_points_device(c, h, c->in_scalars.p, n_msm, terms, c->outs.p, c->flags.p);
     if (rc) return rc;
-    std::vector<uint8_t> st(n_msm);
-    CK(c, cudaMemcpyAsync(outs, c->outs.p, n_msm * 32, cudaMemcpyDeviceToHost, c->stream));
-    CK(c, cudaMemcpyAsync(st.data(), c->flags.p, n_msm, cudaMemcpyDeviceToHost, c->stream));
-    CK(c, cudaStreamSynchronize(c->stream));
-    if (status) memcpy(status, st.data(), n_msm);
-    return BP_OK;
+    return msm_copy_out(c, n_msm, outs, status);
 }
 
 // ---------------------------------------------------------------------------------------------- generators
-static int gens_alloc(bp_ctx *c, size_t cap, size_t parties, bp_gens **out) {
-    if (!c || !out || cap == 0 || parties == 0) return BP_ERR_INVALID_ARGUMENT;
-    CK(c, cudaSetDevice(c->device));
-    bp_gens *g = new bp_gens();
-    g->ctx = c; g->cap = cap; g->parties = parties; g->n_points = 2 + 2 * cap * parties;
-    cudaError_t e = cudaMalloc((void **)&g->d_table, g->n_points * sizeof(ge_niels));
-    if (e != cudaSuccess) { c->err = std::string("cudaMalloc(gens): ") + cudaGetErrorString(e); delete g; return BP_ERR_CUDA; }
-    *out = g;
+int bp_gens_create_empty(bp_ctx *c, size_t cap, size_t parties, bp_gens **out) {
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    std::unique_ptr<bp_gens> g;
+    int rc = gens_alloc(c, cap, parties, g);
+    if (rc) return rc;
+    *out = g.release();
     return BP_OK;
 }
-int bp_gens_create_empty(bp_ctx *c, size_t cap, size_t parties, bp_gens **out) { return gens_alloc(c, cap, parties, out); }
 
 int bp_gens_create(bp_ctx *c, size_t cap, size_t parties, bp_gens **out) {
-    int rc = gens_alloc(c, cap, parties, out);
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    std::unique_ptr<bp_gens> g;
+    int rc = gens_alloc(c, cap, parties, g);
     if (rc) return rc;
-    bp_gens *g = *out;
     // ristretto255 basepoint, compressed (RISTRETTO_BASEPOINT_COMPRESSED)
     static const uint8_t BASEPOINT[32] = {0xe2, 0xf2, 0xae, 0x0a, 0x6a, 0xbc, 0x4e, 0x71, 0xa8, 0x84, 0xa9, 0x61, 0xc5, 0x00, 0x51, 0x5f,
                                           0x58, 0xe3, 0x0b, 0x6a, 0xa5, 0x82, 0xdd, 0x8d, 0xb6, 0xa6, 0x59, 0x45, 0xe0, 0x8d, 0x2d, 0x76};
@@ -513,216 +768,31 @@ int bp_gens_create(bp_ctx *c, size_t cap, size_t parties, bp_gens **out) {
     cudaStream_t s = c->stream;
     CK(c, cudaMemcpyAsync(c->in_points.p, uni.data(), uni.size(), cudaMemcpyHostToDevice, s));
     CK(c, cudaMemcpyAsync(c->in_scalars.p, BASEPOINT, 32, cudaMemcpyHostToDevice, s));
-    LAUNCH(c, KID_FROM_UNIFORM, k_from_uniform<<<blocks_for(g->n_points, 128), 128, 0, s>>>(c->in_points.as<uint8_t>(), g->n_points, g->d_table, nullptr));
-    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<1, 128, 0, s>>>(c->in_scalars.as<uint8_t>(), 1, g->d_table + 1, nullptr));
+    LAUNCH(c, KID_FROM_UNIFORM, k_from_uniform<<<blocks_for(g->n_points, 128), 128, 0, s>>>(c->in_points.as<uint8_t>(), g->n_points, g->d_table(), nullptr));
+    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<1, 128, 0, s>>>(c->in_scalars.as<uint8_t>(), 1, g->d_table() + 1, nullptr));
     CK(c, cudaStreamSynchronize(s));
+    *out = g.release();
     return BP_OK;
 }
-void bp_gens_destroy(bp_gens *g) { if (!g) return; cudaSetDevice(g->ctx->device); cudaFree(g->d_table); delete g; }
+void bp_gens_destroy(bp_gens *g) { if (!g) return; cudaSetDevice(g->ctx->device); delete g; }
 int bp_gens_device_table(bp_gens *g, void **d_table, size_t *bytes) {
     if (!g || !d_table || !bytes) return BP_ERR_INVALID_ARGUMENT;
-    *d_table = g->d_table; *bytes = g->n_points * sizeof(ge_niels); return BP_OK;
+    *d_table = g->table.p; *bytes = g->n_points * sizeof(ge_niels); return BP_OK;
 }
 int bp_gens_get(bp_gens *g, int which, size_t party, size_t index, uint8_t out[32]) {
     if (!g || !out) return BP_ERR_INVALID_ARGUMENT;
     bp_ctx *c = g->ctx; size_t slot;
     if (which == 2) slot = 1; else if (which == 3) slot = 0;
-    else if ((which == 0 || which == 1) && party < g->parties && index < g->cap) slot = 2 + ((size_t)which * g->parties + party) * g->cap + index;
+    else if ((which == 0 || which == 1) && party < g->parties && index < g->cap) slot = gens_slot<size_t>(which, party, index, g->cap, g->parties);
     else return BP_ERR_INVALID_ARGUMENT;
     CK(c, cudaSetDevice(c->device)); CK(c, c->outs.ensure(32));
-    LAUNCH(c, KID_SMALL, k_niels_to_compressed<<<1, 32, 0, c->stream>>>(g->d_table + slot, 1, c->outs.as<uint8_t>()));
+    LAUNCH(c, KID_SMALL, k_niels_to_compressed<<<1, 32, 0, c->stream>>>(g->d_table() + slot, 1, c->outs.as<uint8_t>()));
     CK(c, cudaMemcpyAsync(out, c->outs.p, 32, cudaMemcpyDeviceToHost, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
     return BP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------- range proofs
-// Parameter checks of verify_multiple_with_rng (mod.rs:358-366) and of from_bytes / verification_scalars
-// that depend only on (proof_len, n, m): one verdict for the whole call, or BP_PROOF_OK to go on.
-static uint8_t rp_param_verdict(const bp_gens *gens, size_t proof_len, size_t n, size_t m, rp_geom *g) {
-    if (proof_len % 32 != 0 || proof_len < 7 * 32) return BP_PROOF_FORMAT_ERROR;                 // mod.rs:498-503
-    size_t ne = (proof_len - 7 * 32) / 32;
-    if (ne < 2 || (ne - 2) % 2 != 0 || (ne - 2) / 2 >= 32) return BP_PROOF_FORMAT_ERROR;         // inner_product_proof.rs:375-388
-    size_t k = (ne - 2) / 2;
-    if (!(n == 8 || n == 16 || n == 32 || n == 64)) return BP_PROOF_INVALID_BITSIZE;
-    if (gens->cap < n || gens->parties < m) return BP_PROOF_INVALID_GENERATORS_LENGTH;
-    if (m == 0 || n * m != ((size_t)1 << k) || k > BP_MAX_LG_N) return BP_PROOF_VERIFICATION_ERROR;   // inner_product_proof.rs:204-211
-    g->n = (uint32_t)n; g->m = (uint32_t)m; g->k = (uint32_t)k; g->N = (uint32_t)(n * m);
-    g->D = (uint32_t)(4 + 2 * k + m); g->S = 2 + 2 * g->N; g->proof_len = (uint32_t)proof_len;
-    return BP_PROOF_OK;
-}
-static bool rp_set_group(rp_geom *g, size_t count, size_t n_batches) {
-    if (count == 0 || n_batches == 0 || n_batches > BP_MAX_GROUP_BATCHES || count >= (1u << 24)) return false;
-    size_t T = (size_t)g->S + count * g->D;
-    if (T * n_batches >= (1u << 31) || count * n_batches >= (1u << 24)) return false;
-    g->count = (uint32_t)count; g->nbatch = (uint32_t)n_batches; g->T = (uint32_t)T;
-    return true;
-}
-
-// every arena of one launch group (grow-only); after this nothing on the verification path allocates
-static int rp_ensure(bp_ctx *c, const rp_geom &g) {
-    size_t total = (size_t)g.count * g.nbatch, TT = (size_t)g.T * g.nbatch;
-    CK(c, c->rp_par.ensure(sizeof(rp_params)));
-    CK(c, c->rp_contrib.ensure(total * g.S * sizeof(sc))); CK(c, c->rp_scalars.ensure(TT * 32));
-    CK(c, c->rp_part.ensure((size_t)g.nbatch * ((g.count + RP_CHUNK - 1) / RP_CHUNK) * g.S * sizeof(sc)));
-    CK(c, c->rp_status.ensure(total * 4)); CK(c, c->rp_decbad.ensure(total * 4)); CK(c, c->rp_niels.ensure(total * g.D * sizeof(ge_niels)));
-    CK(c, c->rp_pidx.ensure(TT * 4)); CK(c, c->rp_offsets.ensure(((size_t)g.nbatch + 1) * 4)); CK(c, c->rp_results.ensure((size_t)g.nbatch * sizeof(ge_ext)));
-    CK(c, c->rp_batch_ok.ensure((size_t)g.nbatch * 4)); CK(c, c->rp_combined.ensure((size_t)g.nbatch * 4));
-    CK(c, c->rp_chal.ensure(total * sizeof(rp_head))); CK(c, c->rp_tabs.ensure(total * rp_tab_size(g.k, g.m) * sizeof(sc)));
-    CK(c, c->rp_raw.ensure(total * (RP_RAW_U + g.k) * 64));
-    if (!c->h_verdict || c->h_verdict_cap < total) {
-        if (c->h_verdict) cudaFreeHost(c->h_verdict);
-        c->h_verdict = nullptr; c->h_verdict_cap = 0;
-        CK(c, cudaMallocHost((void **)&c->h_verdict, total * 4));
-        c->h_verdict_cap = total;
-    }
-    if (!c->pow2_tab.p) {            // 2^e (e < 64) in Montgomery form, computed once per context with the host build of sc.cuh
-        std::vector<sc> tab(64);
-        for (int e = 0; e < 64; e++) tab[e] = sc_mont_from_u64(1ULL << e);
-        CK(c, c->pow2_tab.ensure(64 * sizeof(sc)));
-        CK(c, cudaMemcpyAsync(c->pow2_tab.p, tab.data(), 64 * sizeof(sc), cudaMemcpyHostToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream));
-    }
-    return msm_ensure(c, c->ar_rp, msm_make_plan((uint32_t)TT, g.nbatch, 0));
-}
-// signature of every device address the launch sequence of a group bakes into its graph: a regrown (moved) arena invalidates the graph
-static uint64_t rp_ptr_signature(const bp_ctx *c) {
-    const DevBuf *bufs[] = {&c->rp_par, &c->rp_contrib, &c->rp_part, &c->rp_scalars, &c->rp_status, &c->rp_decbad, &c->rp_niels, &c->rp_pidx, &c->rp_offsets, &c->rp_results, &c->rp_batch_ok, &c->rp_combined,
-                            &c->rp_chal, &c->rp_tabs, &c->rp_raw, &c->pow2_tab, &c->ar_rp.counts, &c->ar_rp.starts, &c->ar_rp.cursor, &c->ar_rp.order, &c->ar_rp.sorted, &c->ar_rp.buckets, &c->ar_rp.wsums};
-    uint64_t h = 1469598103934665603ULL;
-    for (const DevBuf *b : bufs) { h ^= (uint64_t)(uintptr_t)b->p; h *= 1099511628211ULL; }
-    return h;
-}
-// term -> point map and MSM offsets of the combined MSMs: depend only on the geometry, rebuilt when it changes
-static int rp_build_maps(bp_ctx *c, bp_gens *gens, const rp_geom &g) {
-    size_t key[6] = {g.n, g.m, g.count, g.nbatch, gens->cap, gens->parties};
-    if (memcmp(key, c->pidx_key, sizeof key) == 0) return BP_OK;
-    cudaStream_t s = c->stream;
-    LAUNCH(c, KID_SMALL, k_rp_point_idx<<<blocks_for((size_t)g.T * g.nbatch, 256), 256, 0, s>>>(g, (uint32_t)gens->cap, (uint32_t)gens->parties, g.count, 0, 0, c->rp_pidx.as<uint32_t>()));
-    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)g.nbatch + 1, 256), 256, 0, s>>>(g.nbatch, g.T, c->rp_offsets.as<uint32_t>()));
-    memcpy(c->pidx_key, key, sizeof key);
-    return BP_OK;
-}
-// upload the per-call parameter block through the pinned staging ring, so that the asynchronous upload never reads caller
-// memory after the entry point returns
-static int rp_upload_params(bp_ctx *c, const uint8_t *h_transcript, const uint8_t *seed, const uint8_t *d_proofs, const uint8_t *d_commit, uint32_t *d_verdict) {
-    unsigned slot = c->stage_next++ % bp_ctx::STAGE_SLOTS;
-    CK(c, cudaEventSynchronize(c->stage_ev[slot]));                          // the upload that last used this slot is done
-    rp_params *par = reinterpret_cast<rp_params *>(c->h_stage + 512 * slot);
-    memset(par, 0, sizeof *par);
-    memcpy(par->tstate, h_transcript, BP_TRANSCRIPT_BYTES);
-    if (seed) memcpy(par->seed, seed, 32);
-    else if (getrandom(par->seed, 32, 0) != 32) { c->err = "getrandom failed"; return BP_ERR_CUDA; }
-    par->proofs = d_proofs; par->commitments = d_commit; par->verdict = d_verdict;
-    CK(c, cudaMemcpyAsync(c->rp_par.p, par, sizeof *par, cudaMemcpyHostToDevice, c->stream));
-    CK(c, cudaEventRecord(c->stage_ev[slot], c->stream));
-    return BP_OK;
-}
-
-// The launch sequence of one group, launches only (no allocation, no synchronisation: capturable).  Two branches: the
-// decompressions need nothing but the proof bytes and run beside the transcript replay and the head.
-static int rp_chain(bp_ctx *c, bp_gens *gens, const rp_geom &g) {
-    cudaStream_t s = c->stream, s2 = c->prof_on ? c->stream : c->aux;
-    const uint32_t total = g.count * g.nbatch;
-    const rp_params *par = c->rp_par.as<rp_params>();
-    uint8_t *d_scal = c->rp_scalars.as<uint8_t>();
-    if (s2 != s) { CK(c, cudaEventRecord(c->ev_fork, s)); CK(c, cudaStreamWaitEvent(s2, c->ev_fork, 0)); }
-    CK(c, cudaMemsetAsync(c->rp_decbad.p, 0, (size_t)total * 4, s2));
-    {   // branch 2
-        cudaStream_t keep = c->stream; c->stream = s2;          // LAUNCH brackets its events on ctx->stream
-        int rc = [&]() -> int {
-            const size_t dec_smem = (size_t)(RP_DEC_THREADS / g.D + 2) * (g.proof_len + 32 * g.m);
-            LAUNCH(c, KID_RP_DECOMPRESS, k_rp_decompress<<<blocks_for((size_t)total * g.D, RP_DEC_THREADS), RP_DEC_THREADS, dec_smem, s2>>>(par, g, total, c->rp_niels.as<ge_niels>(), c->rp_decbad.as<uint32_t>()));
-            return BP_OK;
-        }();
-        c->stream = keep;
-        if (rc) return rc;
-    }
-    if (s2 != s) CK(c, cudaEventRecord(c->ev_join, s2));
-    LAUNCH(c, KID_RP_TRANSCRIPT, k_rp_transcript<<<blocks_for(total, RP_TR_THREADS), RP_TR_THREADS, 0, s>>>(par, g, total, c->rp_raw.as<uint8_t>(), c->rp_status.as<uint32_t>()));
-    LAUNCH(c, KID_RP_HEAD, k_rp_head_seq<<<blocks_for(total, 32), 32, 0, s>>>(par, g, c->rp_raw.as<uint8_t>(), total, c->rp_chal.as<rp_head>(), c->rp_tabs.as<sc>(),
-                                                                                  c->pow2_tab.as<sc>(), c->rp_status.as<uint32_t>()));
-    if (s2 != s) CK(c, cudaStreamWaitEvent(s, c->ev_join, 0));
-    const uint32_t nchunks = (g.count + RP_CHUNK - 1) / RP_CHUNK;
-    LAUNCH(c, KID_RP_SCALARS, k_rp_scalars_sum<<<g.nbatch * nchunks, (unsigned)std::min<uint32_t>(128, std::max<uint32_t>(32, g.N)), 0, s>>>(g, c->rp_chal.as<rp_head>(), c->rp_tabs.as<sc>(),
-                                                                                  c->rp_decbad.as<uint32_t>(), c->rp_part.as<sc>(), d_scal));
-    LAUNCH(c, KID_RP_STATIC_REDUCE, k_rp_static_sum<<<dim3(g.S, g.nbatch), 32, 0, s>>>(c->rp_part.as<sc>(), g, d_scal));
-    MsmArgs a{d_scal, c->rp_offsets.as<uint32_t>(), g.nbatch, g.T * g.nbatch, c->rp_pidx.as<uint32_t>(), gens->d_table, c->rp_niels.as<ge_niels>(), nullptr, 0};
-    int rc = msm_launch(c, c->ar_rp, a, msm_make_plan(a.T, a.n_msm, 0), c->rp_results.as<ge_ext>());
-    if (rc) return rc;
-    LAUNCH(c, KID_SMALL, k_rp_verdict_batch<<<g.nbatch, 256, 0, s>>>(c->rp_status.as<uint32_t>(), c->rp_decbad.as<uint32_t>(), c->rp_results.as<ge_ext>(), g, par,
-                                                                      c->rp_batch_ok.as<uint32_t>(), c->rp_combined.as<uint32_t>()));
-    return BP_OK;
-}
-
-static bool rp_graph_matches(const bp_ctx *c, const bp_gens *gens, const rp_geom &g) {
-    size_t key[6] = {g.n, g.m, g.count, g.nbatch, (size_t)(uintptr_t)gens->d_table, g.proof_len};      // the table address is a kernel argument of the captured nodes
-    return c->graph && memcmp(key, c->graph_key, sizeof key) == 0 && c->graph_sig == rp_ptr_signature(c);
-}
-// queue everything up to the verdicts; d_proofs / d_commitments are device pointers
-static int rp_verify_queue(bp_ctx *c, bp_gens *gens, const rp_geom &g, const uint8_t *d_proofs, const uint8_t *d_commit,
-                           const uint8_t *h_transcript, const uint8_t *seed, uint32_t *d_verdict) {
-    const bool use_graph = !c->prof_on && rp_graph_matches(c, gens, g);
-    if (!use_graph) { int rc = rp_ensure(c, g); if (rc) return rc; }
-    int rc = rp_build_maps(c, gens, g);          // another geometry may have used the context since: the maps follow the key
-    if (rc) return rc;
-    rc = rp_upload_params(c, h_transcript, seed, d_proofs, d_commit, d_verdict);
-    if (rc) return rc;
-    if (use_graph) { CK(c, cudaGraphLaunch(c->graph, c->stream)); c->launches += c->graph_launches; return BP_OK; }
-    return rp_chain(c, gens, g);
-}
-
-// per-proof re-check of the proofs [p0, p0 + count) of a group: count independent MSMs of S + D terms
-static int rp_fallback_range(bp_ctx *c, bp_gens *gens, const rp_geom &g, uint32_t p0, uint32_t count, uint32_t *d_verdict) {
-    cudaStream_t s = c->stream;
-    uint32_t row = g.S + g.D; size_t T = (size_t)count * row;
-    if (T >= (1u << 31)) { c->err = "fallback batch too large"; return BP_ERR_INVALID_ARGUMENT; }
-    CK(c, c->fb_scalars.ensure(T * 32)); CK(c, c->fb_pidx.ensure(T * 4)); CK(c, c->fb_offsets.ensure(((size_t)count + 1) * 4));
-    CK(c, c->results.ensure((size_t)count * sizeof(ge_ext)));
-    uint32_t batch = p0 / g.count, q0 = p0 % g.count;
-    const uint8_t *dyn = c->rp_scalars.as<uint8_t>() + ((size_t)batch * g.T + g.S + (size_t)q0 * g.D) * 32;
-    LAUNCH(c, KID_SMALL, k_rp_expand_scalars<<<blocks_for(T, 128), 128, 0, s>>>(c->rp_contrib.as<sc>() + (size_t)p0 * g.S, dyn, g, count, c->fb_scalars.as<uint8_t>()));
-    LAUNCH(c, KID_SMALL, k_rp_point_idx<<<blocks_for(T, 256), 256, 0, s>>>(g, (uint32_t)gens->cap, (uint32_t)gens->parties, count, 1, p0 * g.D, c->fb_pidx.as<uint32_t>()));
-    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)count + 1, 256), 256, 0, s>>>(count, row, c->fb_offsets.as<uint32_t>()));
-    MsmArgs a{c->fb_scalars.as<uint8_t>(), c->fb_offsets.as<uint32_t>(), count, (uint32_t)T, c->fb_pidx.as<uint32_t>(), gens->d_table, c->rp_niels.as<ge_niels>(), nullptr, 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
-    if (rc) return rc;
-    LAUNCH(c, KID_SMALL, k_rp_verdict_proofs<<<blocks_for(count, 128), 128, 0, s>>>(c->rp_status.as<uint32_t>() + p0, c->rp_decbad.as<uint32_t>() + p0, c->results.as<ge_ext>(), count, d_verdict + p0));
-    return BP_OK;
-}
-// A batch whose combined check failed.  Level 1: one combined MSM per chunk of RP_CHUNK proofs, from the partial sums the main path
-// already holds (one pipeline pass over the batch's ~T terms).  Level 2: the proofs of the failing chunks, each with its own MSM
-// (mod.rs:421-447 per proof).  One bad proof in 1024 costs two small passes instead of 1024 147-term MSMs.
-static int rp_verify_fallback(bp_ctx *c, bp_gens *gens, const rp_geom &g, uint32_t batch, uint32_t *d_verdict, bool *contrib_ready) {
-    cudaStream_t s = c->stream;
-    const uint32_t nch = (g.count + RP_CHUNK - 1) / RP_CHUNK, row = g.S + RP_CHUNK * g.D, p0 = batch * g.count;
-    size_t T = (size_t)nch * row;
-    if (T >= (1u << 31)) { c->err = "fallback batch too large"; return BP_ERR_INVALID_ARGUMENT; }
-    CK(c, c->fb_scalars.ensure(T * 32)); CK(c, c->fb_pidx.ensure(T * 4)); CK(c, c->fb_offsets.ensure(((size_t)nch + 1) * 4));
-    CK(c, c->results.ensure((size_t)nch * sizeof(ge_ext))); CK(c, c->flags.ensure((size_t)nch * 4));
-    LAUNCH(c, KID_SMALL, k_rp_chunk_rows<<<blocks_for(T, 128), 128, 0, s>>>(c->rp_part.as<sc>() + (size_t)batch * nch * g.S, c->rp_scalars.as<uint8_t>() + ((size_t)batch * g.T + g.S) * 32, g,
-                                                                              (uint32_t)gens->cap, (uint32_t)gens->parties, p0 * g.D, c->fb_scalars.as<uint8_t>(), c->fb_pidx.as<uint32_t>()));
-    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)nch + 1, 256), 256, 0, s>>>(nch, row, c->fb_offsets.as<uint32_t>()));
-    MsmArgs a{c->fb_scalars.as<uint8_t>(), c->fb_offsets.as<uint32_t>(), nch, (uint32_t)T, c->fb_pidx.as<uint32_t>(), gens->d_table, c->rp_niels.as<ge_niels>(), nullptr, 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
-    if (rc) return rc;
-    LAUNCH(c, KID_SMALL, k_rp_verdict_chunks<<<blocks_for(g.count, 128), 128, 0, s>>>(c->rp_status.as<uint32_t>() + p0, c->rp_decbad.as<uint32_t>() + p0, c->results.as<ge_ext>(), g.count,
-                                                                                      d_verdict + p0, c->flags.as<uint32_t>()));
-    std::vector<uint32_t> ok(nch);
-    CK(c, cudaMemcpyAsync(ok.data(), c->flags.p, (size_t)nch * 4, cudaMemcpyDeviceToHost, s)); CK(c, cudaStreamSynchronize(s));
-    uint32_t nfail = 0; for (uint32_t v : ok) nfail += v ? 0 : 1;
-    if (nfail == 0) return BP_OK;       // cannot happen when the batch's combination failed, short of a 2^-128 cancellation between chunk weights
-    if (!*contrib_ready) {   // the combined path keeps only sums: the per-proof static-term scalars are produced here, on the reject path (whole group; idempotent)
-        const uint32_t total = g.count * g.nbatch;
-        LAUNCH(c, KID_RP_SCALARS, k_rp_scalars<<<blocks_for((size_t)total * (g.N + g.D), 128), 128, 0, s>>>(g, c->rp_chal.as<rp_head>(), c->rp_tabs.as<sc>(), c->rp_decbad.as<uint32_t>(), total,
-                                                                                                            c->rp_contrib.as<sc>(), c->rp_scalars.as<uint8_t>()));
-        *contrib_ready = true;
-    }
-    if (nfail > 4) return rp_fallback_range(c, gens, g, p0, g.count, d_verdict);      // many bad chunks: one pass over the whole batch
-    for (uint32_t ch = 0; ch < nch; ch++)
-        if (!ok[ch]) { rc = rp_fallback_range(c, gens, g, p0 + ch * RP_CHUNK, std::min<uint32_t>(RP_CHUNK, g.count - ch * RP_CHUNK), d_verdict); if (rc) return rc; }
-    return BP_OK;
-}
-
 int bp_rangeproof_verify_reserve(bp_ctx *c, bp_gens *gens, size_t n, size_t m, size_t count, size_t n_batches) {
     if (!c || !gens) return BP_ERR_INVALID_ARGUMENT;
     BUSY_CHECK(c);
@@ -748,8 +818,7 @@ int bp_rangeproof_verify_reserve(bp_ctx *c, bp_gens *gens, size_t n, size_t m, s
     e = cudaGraphInstantiate(&c->graph, graph, 0);
     cudaGraphDestroy(graph);
     if (e != cudaSuccess) { c->graph = nullptr; c->err = std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e); return BP_ERR_CUDA; }
-    size_t key[6] = {g.n, g.m, g.count, g.nbatch, (size_t)(uintptr_t)gens->d_table, g.proof_len};      // the table address is a kernel argument of the captured nodes
-    memcpy(c->graph_key, key, sizeof key); c->graph_sig = rp_ptr_signature(c);
+    c->graph_key = rp_graph_key(gens, g); c->graph_sig = c->rp.signature();
     // one untimed pass so that the first real call finds module loading, the graph upload and the L2 working set done
     std::vector<uint8_t> zt(BP_TRANSCRIPT_BYTES, 0);
     CK(c, cudaMemsetAsync(c->rp_proofs.p, 0, (size_t)g.count * g.nbatch * g.proof_len, c->stream)); CK(c, cudaMemsetAsync(c->rp_commit.p, 0, (size_t)g.count * g.nbatch * m * 32, c->stream));
@@ -777,9 +846,9 @@ int bp_rangeproof_verify_group_begin(bp_ctx *c, bp_gens *gens, const uint8_t *tr
     CK(c, cudaMemcpyAsync(c->rp_commit.p, commitments, total * m * 32, cudaMemcpyHostToDevice, c->stream));
     int rc = rp_verify_queue(c, gens, g, c->rp_proofs.as<uint8_t>(), c->rp_commit.as<uint8_t>(), transcript, seed, c->rp_verdict.as<uint32_t>());
     if (rc) return rc;
-    CK(c, cudaMemcpyAsync(c->h_verdict, c->rp_verdict.p, total * 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(c, cudaMemcpyAsync(c->h_flag, c->rp_combined.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(c, cudaMemcpyAsync(c->h_flag + BP_MAX_GROUP_BATCHES, c->rp_batch_ok.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaMemcpyAsync(c->h_verdict.p, c->rp_verdict.p, total * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaMemcpyAsync(c->h_flag.p, c->rp.combined.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaMemcpyAsync(c->h_flag.as<uint32_t>() + BP_MAX_GROUP_BATCHES, c->rp.batch_ok.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
     vs.active = true; c->vs = vs;              // only a fully queued verification is pending
     return BP_OK;
 }
@@ -792,17 +861,17 @@ int bp_rangeproof_verify_group_finish(bp_ctx *c, uint8_t *verdicts, uint8_t *bat
     CK(c, cudaStreamSynchronize(c->stream));
     bool redo = false, contrib_ready = false;
     for (uint32_t b = 0; b < vs.g.nbatch; b++)
-        if (c->h_flag[b] == 0) {            // this batch's combined check failed: find the offenders (chunks of 32, then proof by proof)
+        if (c->h_flag.as<uint32_t>()[b] == 0) {            // this batch's combined check failed: find the offenders (chunks of 32, then proof by proof)
             int rc = rp_verify_fallback(c, vs.gens, vs.g, b, c->rp_verdict.as<uint32_t>(), &contrib_ready);
             if (rc) return rc;
             redo = true;
         }
     if (redo) {
-        CK(c, cudaMemcpyAsync(c->h_verdict, c->rp_verdict.p, (size_t)vs.total * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(c, cudaMemcpyAsync(c->h_verdict.p, c->rp_verdict.p, (size_t)vs.total * 4, cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
-    for (uint32_t i = 0; i < vs.total; i++) verdicts[i] = (uint8_t)c->h_verdict[i];
-    if (batch_ok) for (uint32_t b = 0; b < vs.g.nbatch; b++) batch_ok[b] = (uint8_t)c->h_flag[BP_MAX_GROUP_BATCHES + b];
+    for (uint32_t i = 0; i < vs.total; i++) verdicts[i] = (uint8_t)c->h_verdict.as<uint32_t>()[i];
+    if (batch_ok) for (uint32_t b = 0; b < vs.g.nbatch; b++) batch_ok[b] = (uint8_t)c->h_flag.as<uint32_t>()[BP_MAX_GROUP_BATCHES + b];
     return BP_OK;
 }
 
@@ -816,7 +885,7 @@ int bp_rangeproof_verify_group_device(bp_ctx *c, bp_gens *gens, const uint8_t *t
     if (pv != BP_PROOF_OK || !rp_set_group(&g, count, n_batches)) return BP_ERR_INVALID_ARGUMENT;
     int rc = rp_verify_queue(c, gens, g, (const uint8_t *)d_proofs, (const uint8_t *)d_commitments, transcript, seed, (uint32_t *)d_verdicts_u32);
     if (rc) return rc;
-    if (h_batch_ok_pinned) CK(c, cudaMemcpyAsync(h_batch_ok_pinned, c->rp_batch_ok.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (h_batch_ok_pinned) CK(c, cudaMemcpyAsync(h_batch_ok_pinned, c->rp.batch_ok.p, (size_t)g.nbatch * 4, cudaMemcpyDeviceToHost, c->stream));
     return BP_OK;
 }
 
@@ -838,11 +907,6 @@ int bp_rangeproof_verify_batch_device(bp_ctx *c, bp_gens *gens, const uint8_t *t
 }
 
 // ---------------------------------------------------------------------------------------------- indexed MSMs and the IPP prover session
-static int check_scalars_canonical(const uint8_t *s, size_t n) {
-    for (size_t i = 0; i < n; i++) if (sc_geq_l(sc_load(s + 32 * i))) return BP_ERR_NONCANONICAL_SCALAR;
-    return BP_OK;
-}
-
 int bp_msm_indexed_batch(bp_ctx *c, bp_gens *gens, const uint8_t *scalars, const uint32_t *point_idx, const uint8_t *dyn_points, size_t n_dyn,
                          const uint64_t *offsets, size_t n_msm, uint8_t *outs, uint8_t *status) {
     if (!c || !offsets || !outs || n_msm == 0) return BP_ERR_INVALID_ARGUMENT;
@@ -866,18 +930,16 @@ int bp_msm_indexed_batch(bp_ctx *c, bp_gens *gens, const uint8_t *scalars, const
     CK(c, cudaMemcpyAsync(c->ix_pidx.p, point_idx, T * 4, cudaMemcpyHostToDevice, s));
     CK(c, cudaMemsetAsync(c->msm_err.p, 0, (size_t)M * 4, s));
     std::vector<uint8_t> dyn_ok;
-    if (n_dyn) {
+    if (n_dyn) {          // per-point flags, not a failure: an invalid point only poisons the MSMs that use it (below)
         CK(c, c->in_points.ensure(n_dyn * 32)); CK(c, c->niels.ensure(n_dyn * sizeof(ge_niels))); CK(c, c->ok.ensure(n_dyn));
         CK(c, cudaMemcpyAsync(c->in_points.p, dyn_points, n_dyn * 32, cudaMemcpyHostToDevice, s));
         LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(n_dyn, 128), 128, 0, s>>>(c->in_points.as<uint8_t>(), n_dyn, c->niels.as<ge_niels>(), c->ok.as<uint8_t>()));
         dyn_ok.resize(n_dyn);
         CK(c, cudaMemcpyAsync(dyn_ok.data(), c->ok.p, n_dyn, cudaMemcpyDeviceToHost, s));
     }
-    MsmArgs a{c->in_scalars.as<uint8_t>(), c->in_offsets.as<uint32_t>(), M, (uint32_t)T, c->ix_pidx.as<uint32_t>(), gens ? gens->d_table : nullptr, c->niels.as<ge_niels>(), c->msm_err.as<uint32_t>(), 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    MsmArgs a{c->in_scalars.as<uint8_t>(), c->in_offsets.as<uint32_t>(), M, (uint32_t)T, c->ix_pidx.as<uint32_t>(), gens ? gens->d_table() : nullptr, c->niels.as<ge_niels>(), c->msm_err.as<uint32_t>(), 0};
+    int rc = msm_to_bytes(c, a, c->outs.as<uint8_t>(), c->flags.as<uint8_t>());
     if (rc) return rc;
-    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(M, 128), 128, 0, s>>>(c->results.as<ge_ext>(), M, c->outs.as<uint8_t>()));
-    LAUNCH(c, KID_SMALL, k_msm_status<<<blocks_for(M, 128), 128, 0, s>>>(c->msm_err.as<uint32_t>(), M, c->flags.as<uint8_t>()));
     std::vector<uint8_t> st(n_msm);
     CK(c, cudaMemcpyAsync(outs, c->outs.p, n_msm * 32, cudaMemcpyDeviceToHost, s));
     CK(c, cudaMemcpyAsync(st.data(), c->flags.p, n_msm, cudaMemcpyDeviceToHost, s));
@@ -891,60 +953,25 @@ int bp_msm_indexed_batch(bp_ctx *c, bp_gens *gens, const uint8_t *scalars, const
     return BP_OK;
 }
 
-}  // extern "C"
-
-struct bp_ipp {
-    bp_ctx *ctx = nullptr; uint32_t N = 0; ge_niels *pts = nullptr;     // [G (N) | H (N) | Q]
-    DevBuf scal, idx, offs;
-};
-
-extern "C" {
-
-static int ipp_alloc(bp_ctx *c, size_t N, bp_ipp **out) {
-    if (!c || !out || N == 0 || (N & (N - 1)) || N >= (1u << 24)) return BP_ERR_INVALID_ARGUMENT;      // power of two (inner_product_proof.rs:67)
-    CK(c, cudaSetDevice(c->device));
-    bp_ipp *s = new bp_ipp(); s->ctx = c; s->N = (uint32_t)N;
-    cudaError_t e = cudaMalloc((void **)&s->pts, (2 * N + 1) * sizeof(ge_niels));
-    if (e != cudaSuccess) { c->err = std::string("cudaMalloc(ipp): ") + cudaGetErrorString(e); delete s; return BP_ERR_CUDA; }
-    *out = s; return BP_OK;
-}
-int bp_ipp_begin(bp_ctx *c, bp_gens *gens, size_t n, size_t m, const uint8_t Q[32], bp_ipp **out) {
-    if (!gens || !Q || n == 0 || m == 0 || n > gens->cap || m > gens->parties) return BP_ERR_INVALID_ARGUMENT;
-    size_t N = n * m;
-    int rc = ipp_alloc(c, N, out); if (rc) return rc;
-    bp_ipp *s = *out;
-    std::vector<uint32_t> idx(2 * N);
-    for (size_t q = 0; q < N; q++) {          // BulletproofGens::G(n, m) / H(n, m) iterator order (generators.rs:207-259)
-        idx[q] = (uint32_t)(2 + (q / n) * gens->cap + (q % n));
-        idx[N + q] = (uint32_t)(2 + gens->parties * gens->cap + (q / n) * gens->cap + (q % n));
-    }
-    cudaStream_t st = c->stream;
-    CK(c, s->idx.ensure(2 * N * 4)); CK(c, c->in_points.ensure(32)); CK(c, c->ok.ensure(1));
-    CK(c, cudaMemcpyAsync(s->idx.p, idx.data(), 2 * N * 4, cudaMemcpyHostToDevice, st));
-    CK(c, cudaMemcpyAsync(c->in_points.p, Q, 32, cudaMemcpyHostToDevice, st));
-    LAUNCH(c, KID_SMALL, k_gather_niels<<<blocks_for(2 * N, 128), 128, 0, st>>>(gens->d_table, s->idx.as<uint32_t>(), (uint32_t)(2 * N), s->pts));
-    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<1, 128, 0, st>>>(c->in_points.as<uint8_t>(), 1, s->pts + 2 * N, c->ok.as<uint8_t>()));
-    uint8_t ok = 0;
-    CK(c, cudaMemcpyAsync(&ok, c->ok.p, 1, cudaMemcpyDeviceToHost, st)); CK(c, cudaStreamSynchronize(st));
-    if (!ok) { cudaFree(s->pts); delete s; *out = nullptr; return BP_ERR_INVALID_POINT; }
-    return BP_OK;
-}
 int bp_ipp_begin_points(bp_ctx *c, const uint8_t *G, const uint8_t *H, size_t N, const uint8_t Q[32], bp_ipp **out) {
-    if (!G || !H || !Q) return BP_ERR_INVALID_ARGUMENT;
-    int rc = ipp_alloc(c, N, out); if (rc) return rc;
-    bp_ipp *s = *out; cudaStream_t st = c->stream;
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    if (!c || !G || !H || !Q || N == 0 || (N & (N - 1)) || N >= (1u << 24)) return BP_ERR_INVALID_ARGUMENT;      // power of two (inner_product_proof.rs:67)
+    CK(c, cudaSetDevice(c->device));
+    std::unique_ptr<bp_ipp> s(new bp_ipp()); s->ctx = c; s->N = (uint32_t)N;
     size_t n_pts = 2 * N + 1;
-    CK(c, c->in_points.ensure(n_pts * 32)); CK(c, c->ok.ensure(n_pts));
+    CK(c, s->pts.alloc(n_pts * sizeof(ge_niels)));
+    cudaStream_t st = c->stream;
+    CK(c, c->in_points.ensure(n_pts * 32));
     CK(c, cudaMemcpyAsync(c->in_points.p, G, N * 32, cudaMemcpyHostToDevice, st));
     CK(c, cudaMemcpyAsync(c->in_points.as<uint8_t>() + N * 32, H, N * 32, cudaMemcpyHostToDevice, st));
     CK(c, cudaMemcpyAsync(c->in_points.as<uint8_t>() + 2 * N * 32, Q, 32, cudaMemcpyHostToDevice, st));
-    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(n_pts, 128), 128, 0, st>>>(c->in_points.as<uint8_t>(), n_pts, s->pts, c->ok.as<uint8_t>()));
-    std::vector<uint8_t> ok(n_pts);
-    CK(c, cudaMemcpyAsync(ok.data(), c->ok.p, n_pts, cudaMemcpyDeviceToHost, st)); CK(c, cudaStreamSynchronize(st));
-    for (uint8_t v : ok) if (!v) { cudaFree(s->pts); delete s; *out = nullptr; return BP_ERR_INVALID_POINT; }
+    int rc = decompress_checked(c, c->in_points.as<uint8_t>(), n_pts, s->pts.as<ge_niels>());
+    if (rc) return rc;
+    *out = s.release();
     return BP_OK;
 }
-void bp_ipp_end(bp_ipp *s) { if (!s) return; cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); cudaFree(s->pts); s->scal.release(); s->idx.release(); s->offs.release(); delete s; }
+void bp_ipp_end(bp_ipp *s) { if (!s) return; cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); delete s; }
 
 // one round's two MSMs: L = <sL[0..h), G_R> + <sL[h..2h), H_L> + sL[2h] Q ;  R = <sR[0..h), G_L> + <sR[h..2h), H_R> + sR[2h] Q
 // (inner_product_proof.rs:87-113,153-163); h = n_half = current length / 2
@@ -968,10 +995,9 @@ int bp_ipp_lr(bp_ipp *s, size_t n_half, const uint8_t *scalars_L, const uint8_t 
     CK(c, cudaMemcpyAsync(s->scal.as<uint8_t>() + per * 32, scalars_R, per * 32, cudaMemcpyHostToDevice, st));
     CK(c, cudaMemcpyAsync(s->idx.p, idx.data(), 2 * per * 4, cudaMemcpyHostToDevice, st));
     CK(c, cudaMemcpyAsync(s->offs.p, offs.data(), 12, cudaMemcpyHostToDevice, st));
-    MsmArgs a{s->scal.as<uint8_t>(), s->offs.as<uint32_t>(), 2, (uint32_t)(2 * per), s->idx.as<uint32_t>(), nullptr, s->pts, nullptr, 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    MsmArgs a{s->scal.as<uint8_t>(), s->offs.as<uint32_t>(), 2, (uint32_t)(2 * per), s->idx.as<uint32_t>(), nullptr, s->pts.as<ge_niels>(), nullptr, 0};
+    int rc = msm_to_bytes(c, a, c->outs.as<uint8_t>(), nullptr);
     if (rc) return rc;
-    LAUNCH(c, KID_COMPRESS, k_compress<<<1, 128, 0, st>>>(c->results.as<ge_ext>(), 2, c->outs.as<uint8_t>()));
     uint8_t lr[64];
     CK(c, cudaMemcpyAsync(lr, c->outs.p, 64, cudaMemcpyDeviceToHost, st)); CK(c, cudaStreamSynchronize(st));
     memcpy(L_out, lr, 32); memcpy(R_out, lr + 32, 32);
@@ -990,106 +1016,56 @@ int bp_ipp_fold(bp_ipp *s, size_t n_half, const uint8_t *g_lo, const uint8_t *g_
     for (int k = 0; k < 4; k++) CK(c, cudaMemcpyAsync(s->scal.as<uint8_t>() + (size_t)k * cnt * 32, arrs[k], cnt * 32, cudaMemcpyHostToDevice, st));
     uint32_t stride = per_index ? 32 : 0;
     const uint8_t *d = s->scal.as<uint8_t>();
-    LAUNCH(c, KID_IPP_FOLD, k_ipp_fold<<<blocks_for(h, 64), 64, 0, st>>>(s->pts, (uint32_t)h, d, d + cnt * 32, stride));
-    LAUNCH(c, KID_IPP_FOLD, k_ipp_fold<<<blocks_for(h, 64), 64, 0, st>>>(s->pts + s->N, (uint32_t)h, d + 2 * cnt * 32, d + 3 * cnt * 32, stride));
+    ge_niels *pts = s->pts.as<ge_niels>();
+    LAUNCH(c, KID_IPP_FOLD, k_ipp_fold<<<blocks_for(h, 64), 64, 0, st>>>(pts, (uint32_t)h, d, d + cnt * 32, stride));
+    LAUNCH(c, KID_IPP_FOLD, k_ipp_fold<<<blocks_for(h, 64), 64, 0, st>>>(pts + s->N, (uint32_t)h, d + 2 * cnt * 32, d + 3 * cnt * 32, stride));
     CK(c, cudaStreamSynchronize(st));          // the scalar staging buffer is reused by the next round
     return BP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------- inner-product prover, device-resident state
-}  // extern "C"
-struct bp_ippx {
-    bp_ctx *ctx = nullptr; uint32_t N = 0, B = 0, n = 0;
-    const ge_niels *d_static = nullptr; ge_niels *own_pts = nullptr;      // the gens table, or the session's own [G (N) | H (N)]
-    ge_niels *d_q = nullptr;                                               // B points Q
-    DevBuf a, b, cG, cH, gidx, hidx, scal, pidx, offs, in, outs;
-};
-extern "C" {
-static void ippx_free(bp_ippx *s);
-static int ippx_alloc(bp_ctx *c, size_t N, size_t B, bp_ippx **out) {
-    if (!c || !out || N == 0 || (N & (N - 1)) || B == 0 || 2 * B * (N + 1) >= (1u << 31)) return BP_ERR_INVALID_ARGUMENT;      // power of two (inner_product_proof.rs:67)
-    BUSY_CHECK(c);
-    CK(c, cudaSetDevice(c->device));
-    bp_ippx *s = new bp_ippx(); s->ctx = c; s->N = (uint32_t)N; s->B = (uint32_t)B; s->n = (uint32_t)N;
-    size_t BN = B * N;
-    cudaError_t e = cudaMalloc((void **)&s->d_q, B * sizeof(ge_niels));
-    if (e != cudaSuccess) { c->err = std::string("cudaMalloc(ippx): ") + cudaGetErrorString(e); delete s; return BP_ERR_CUDA; }
-    int rc = [&]() -> int {
-        for (DevBuf *b : {&s->a, &s->b, &s->cG, &s->cH}) CK(c, b->ensure(BN * sizeof(sc)));
-        CK(c, s->gidx.ensure(N * 4)); CK(c, s->hidx.ensure(N * 4)); CK(c, s->scal.ensure(2 * B * (N + 1) * 32)); CK(c, s->pidx.ensure(2 * B * (N + 1) * 4));
-        CK(c, s->offs.ensure((2 * B + 1) * 4)); CK(c, s->in.ensure(std::max<size_t>(4 * BN * 32, 64 * B))); CK(c, s->outs.ensure(64 * B));
-        return BP_OK;
-    }();
-    if (rc) { ippx_free(s); return rc; }
-    *out = s; return BP_OK;
-}
-static void ippx_free(bp_ippx *s) {
-    cudaFree(s->d_q); if (s->own_pts) cudaFree(s->own_pts);
-    for (DevBuf *b : {&s->a, &s->b, &s->cG, &s->cH, &s->gidx, &s->hidx, &s->scal, &s->pidx, &s->offs, &s->in, &s->outs}) b->release();
-    delete s;
-}
-// common tail of the two begin forms: Q points, scalar vectors (B x N canonical scalars each; Gf / Hf may be NULL = all ones)
-static int ippx_load(bp_ippx *s, const uint8_t *Q, const uint8_t *Gf, const uint8_t *Hf, const uint8_t *a, const uint8_t *b) {
-    bp_ctx *c = s->ctx; cudaStream_t st = c->stream; size_t BN = (size_t)s->B * s->N;
-    for (const uint8_t *v : {a, b}) if (check_scalars_canonical(v, BN)) return BP_ERR_NONCANONICAL_SCALAR;
-    for (const uint8_t *v : {Gf, Hf}) if (v && check_scalars_canonical(v, BN)) return BP_ERR_NONCANONICAL_SCALAR;
-    uint8_t *din = s->in.as<uint8_t>();
-    CK(c, cudaMemcpyAsync(din, a, BN * 32, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(din + BN * 32, b, BN * 32, cudaMemcpyHostToDevice, st));
-    if (Gf) CK(c, cudaMemcpyAsync(din + 2 * BN * 32, Gf, BN * 32, cudaMemcpyHostToDevice, st));
-    if (Hf) CK(c, cudaMemcpyAsync(din + 3 * BN * 32, Hf, BN * 32, cudaMemcpyHostToDevice, st));
-    ippx_geom g{s->N, s->B, s->n};
-    LAUNCH(c, KID_SMALL, k_ippx_init<<<blocks_for(BN, 128), 128, 0, st>>>(g, din, din + BN * 32, Gf ? din + 2 * BN * 32 : nullptr, Hf ? din + 3 * BN * 32 : nullptr,
-                                                                         s->a.as<sc>(), s->b.as<sc>(), s->cG.as<sc>(), s->cH.as<sc>()));
-    CK(c, c->in_points.ensure((size_t)s->B * 32)); CK(c, c->ok.ensure(s->B));
-    CK(c, cudaMemcpyAsync(c->in_points.p, Q, (size_t)s->B * 32, cudaMemcpyHostToDevice, st));
-    LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(s->B, 128), 128, 0, st>>>(c->in_points.as<uint8_t>(), s->B, s->d_q, c->ok.as<uint8_t>()));
-    std::vector<uint8_t> ok(s->B);
-    CK(c, cudaMemcpyAsync(ok.data(), c->ok.p, s->B, cudaMemcpyDeviceToHost, st)); CK(c, cudaStreamSynchronize(st));
-    for (uint8_t v : ok) if (!v) return BP_ERR_INVALID_POINT;
-    LAUNCH(c, KID_SMALL, k_fill_offsets<<<blocks_for((size_t)2 * s->B + 1, 256), 256, 0, st>>>(2 * s->B, s->N + 1, s->offs.as<uint32_t>()));
-    return BP_OK;
-}
 int bp_ippx_begin(bp_ctx *c, bp_gens *gens, size_t n, size_t m, size_t n_proofs, const uint8_t *Q, const uint8_t *Gf, const uint8_t *Hf, const uint8_t *a, const uint8_t *b, bp_ippx **out) {
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
     if (!gens || !Q || !a || !b || n == 0 || m == 0 || n > gens->cap || m > gens->parties) return BP_ERR_INVALID_ARGUMENT;
     size_t N = n * m;
-    int rc = ippx_alloc(c, N, n_proofs, out); if (rc) return rc;
-    bp_ippx *s = *out; s->d_static = gens->d_table;
+    std::unique_ptr<bp_ippx> s;
+    int rc = ippx_alloc(c, N, n_proofs, s); if (rc) return rc;
+    s->d_static = gens->d_table();
     std::vector<uint32_t> idx(2 * N);
-    for (size_t q = 0; q < N; q++) {          // BulletproofGens::G(n, m) / H(n, m) iterator order (generators.rs:207-259)
-        idx[q] = (uint32_t)(2 + (q / n) * gens->cap + (q % n));
-        idx[N + q] = (uint32_t)(2 + gens->parties * gens->cap + (q / n) * gens->cap + (q % n));
+    for (size_t q = 0; q < N; q++) {          // BulletproofGens::G(n, m) / H(n, m) iterator order
+        idx[q] = (uint32_t)gens_slot<size_t>(0, q / n, q % n, gens->cap, gens->parties);
+        idx[N + q] = (uint32_t)gens_slot<size_t>(1, q / n, q % n, gens->cap, gens->parties);
     }
-    rc = [&]() -> int {
-        CK(c, cudaMemcpyAsync(s->gidx.p, idx.data(), N * 4, cudaMemcpyHostToDevice, c->stream)); CK(c, cudaMemcpyAsync(s->hidx.p, idx.data() + N, N * 4, cudaMemcpyHostToDevice, c->stream));
-        CK(c, cudaStreamSynchronize(c->stream));
-        return ippx_load(s, Q, Gf, Hf, a, b);
-    }();
-    if (rc) { ippx_free(s); *out = nullptr; }
-    return rc;
+    CK(c, cudaMemcpyAsync(s->gidx.p, idx.data(), N * 4, cudaMemcpyHostToDevice, c->stream)); CK(c, cudaMemcpyAsync(s->hidx.p, idx.data() + N, N * 4, cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    rc = ippx_load(s.get(), Q, Gf, Hf, a, b);
+    if (rc) return rc;
+    *out = s.release();
+    return BP_OK;
 }
 int bp_ippx_begin_points(bp_ctx *c, const uint8_t *G, const uint8_t *H, size_t N, size_t n_proofs, const uint8_t *Q, const uint8_t *Gf, const uint8_t *Hf, const uint8_t *a, const uint8_t *b, bp_ippx **out) {
+    if (!out) return BP_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
     if (!G || !H || !Q || !a || !b) return BP_ERR_INVALID_ARGUMENT;
-    int rc = ippx_alloc(c, N, n_proofs, out); if (rc) return rc;
-    bp_ippx *s = *out; cudaStream_t st = c->stream;
-    cudaError_t e = cudaMalloc((void **)&s->own_pts, 2 * N * sizeof(ge_niels));
-    if (e != cudaSuccess) { c->err = std::string("cudaMalloc(ippx points): ") + cudaGetErrorString(e); ippx_free(s); *out = nullptr; return BP_ERR_CUDA; }
-    s->d_static = s->own_pts;
-    std::vector<uint8_t> ok(2 * N); std::vector<uint32_t> idx(2 * N);
+    std::unique_ptr<bp_ippx> s;
+    int rc = ippx_alloc(c, N, n_proofs, s); if (rc) return rc;
+    cudaStream_t st = c->stream;
+    CK(c, s->own_pts.alloc(2 * N * sizeof(ge_niels)));
+    s->d_static = s->own_pts.as<ge_niels>();
+    std::vector<uint32_t> idx(2 * N);
     for (size_t q = 0; q < 2 * N; q++) idx[q] = (uint32_t)q;
-    rc = [&]() -> int {
-        CK(c, c->in_points.ensure(2 * N * 32)); CK(c, c->ok.ensure(2 * N));
-        CK(c, cudaMemcpyAsync(c->in_points.p, G, N * 32, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(c->in_points.as<uint8_t>() + N * 32, H, N * 32, cudaMemcpyHostToDevice, st));
-        LAUNCH(c, KID_DECOMPRESS, k_decompress<<<blocks_for(2 * N, 128), 128, 0, st>>>(c->in_points.as<uint8_t>(), 2 * N, s->own_pts, c->ok.as<uint8_t>()));
-        CK(c, cudaMemcpyAsync(ok.data(), c->ok.p, 2 * N, cudaMemcpyDeviceToHost, st));
-        CK(c, cudaMemcpyAsync(s->gidx.p, idx.data(), N * 4, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(s->hidx.p, idx.data() + N, N * 4, cudaMemcpyHostToDevice, st));
-        CK(c, cudaStreamSynchronize(st));
-        for (uint8_t v : ok) if (!v) return BP_ERR_INVALID_POINT;
-        return ippx_load(s, Q, Gf, Hf, a, b);
-    }();
-    if (rc) { ippx_free(s); *out = nullptr; }
-    return rc;
+    CK(c, c->in_points.ensure(2 * N * 32));
+    CK(c, cudaMemcpyAsync(c->in_points.p, G, N * 32, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(c->in_points.as<uint8_t>() + N * 32, H, N * 32, cudaMemcpyHostToDevice, st));
+    CK(c, cudaMemcpyAsync(s->gidx.p, idx.data(), N * 4, cudaMemcpyHostToDevice, st)); CK(c, cudaMemcpyAsync(s->hidx.p, idx.data() + N, N * 4, cudaMemcpyHostToDevice, st));
+    rc = decompress_checked(c, c->in_points.as<uint8_t>(), 2 * N, s->own_pts.as<ge_niels>());
+    if (rc) return rc;
+    rc = ippx_load(s.get(), Q, Gf, Hf, a, b);
+    if (rc) return rc;
+    *out = s.release();
+    return BP_OK;
 }
-void bp_ippx_end(bp_ippx *s) { if (!s) return; cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); ippx_free(s); }
+void bp_ippx_end(bp_ippx *s) { if (!s) return; cudaSetDevice(s->ctx->device); cudaStreamSynchronize(s->ctx->stream); delete s; }
 size_t bp_ippx_current_len(const bp_ippx *s) { return s ? s->n : 0; }
 // L and R of the current round for every proof (inner_product_proof.rs:87-113 / 153-163): LR_out = n_proofs x (L | R) compressed; synchronises
 int bp_ippx_round(bp_ippx *s, uint8_t *LR_out) {
@@ -1101,10 +1077,9 @@ int bp_ippx_round(bp_ippx *s, uint8_t *LR_out) {
     LAUNCH(c, KID_SMALL, k_ippx_rows<<<blocks_for((size_t)s->B * s->N, 128), 128, 0, st>>>(g, s->a.as<sc>(), s->b.as<sc>(), s->cG.as<sc>(), s->cH.as<sc>(), s->gidx.as<uint32_t>(), s->hidx.as<uint32_t>(),
                                                                                           s->scal.as<uint8_t>(), s->pidx.as<uint32_t>()));
     CK(c, c->results.ensure((size_t)M * sizeof(ge_ext)));
-    MsmArgs a{s->scal.as<uint8_t>(), s->offs.as<uint32_t>(), M, T, s->pidx.as<uint32_t>(), s->d_static, s->d_q, nullptr, 0};
-    int rc = msm_core(c, a, c->results.as<ge_ext>());
+    MsmArgs a{s->scal.as<uint8_t>(), s->offs.as<uint32_t>(), M, T, s->pidx.as<uint32_t>(), s->d_static, s->d_q.as<ge_niels>(), nullptr, 0};
+    int rc = msm_to_bytes(c, a, s->outs.as<uint8_t>(), nullptr);
     if (rc) return rc;
-    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(M, 128), 128, 0, st>>>(c->results.as<ge_ext>(), M, s->outs.as<uint8_t>()));
     CK(c, cudaMemcpyAsync(LR_out, s->outs.p, (size_t)M * 32, cudaMemcpyDeviceToHost, st)); CK(c, cudaStreamSynchronize(st));
     return BP_OK;
 }
@@ -1168,12 +1143,12 @@ int bp_prof_timeline(bp_ctx *c, bp_ctx *ref, int *kernel_ids, double *start_ms, 
 int bp_gens_table_export(bp_gens *g, void *d_dst) {
     if (!g || !d_dst) return BP_ERR_INVALID_ARGUMENT;
     bp_ctx *c = g->ctx; CK(c, cudaSetDevice(c->device));
-    CK(c, cudaMemcpyAsync(d_dst, g->d_table, g->n_points * sizeof(ge_niels), cudaMemcpyDeviceToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream)); return BP_OK;
+    CK(c, cudaMemcpyAsync(d_dst, g->d_table(), g->n_points * sizeof(ge_niels), cudaMemcpyDeviceToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream)); return BP_OK;
 }
 int bp_gens_table_import(bp_gens *g, const void *d_src) {
     if (!g || !d_src) return BP_ERR_INVALID_ARGUMENT;
     bp_ctx *c = g->ctx; CK(c, cudaSetDevice(c->device));
-    CK(c, cudaMemcpyAsync(g->d_table, d_src, g->n_points * sizeof(ge_niels), cudaMemcpyDeviceToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream)); return BP_OK;
+    CK(c, cudaMemcpyAsync(g->d_table(), d_src, g->n_points * sizeof(ge_niels), cudaMemcpyDeviceToDevice, c->stream)); CK(c, cudaStreamSynchronize(c->stream)); return BP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------- host helpers

@@ -12,6 +12,10 @@
 
 #define BP_POINT_DYNAMIC 0x80000000u     // point_idx flag: index into the per-call (dynamic) point array
 
+// Slot of G[party][index] (which = 0) or H[party][index] (which = 1) in the generator table [B_blinding, B, G[party][i].., H[party][i]..].
+// BulletproofGens::G(n, m) / H(n, m) visit term q at party q / n, index q % n (generators.rs:207-259).
+template <class U> __host__ __device__ inline U gens_slot(U which, U party, U index, U cap, U parties) { return 2 + (which * parties + party) * cap + index; }
+
 // ------------------------------------------------------------------ vector load/store helpers
 __device__ __forceinline__ void ld32(uint8_t dst[32], const uint8_t *src) {       // 32 B, 16-B aligned
     const uint4 *p = reinterpret_cast<const uint4 *>(src);
@@ -148,13 +152,6 @@ __global__ void __launch_bounds__(128) k_from_uniform(const uint8_t *__restrict_
     ge_ext p = ge_from_uniform(u);
     if (out_comp) { uint8_t s[32]; ge_encode(s, p); st32(out_comp + 32 * i, s); }
     if (out_niels) { fe zi = fe_invert(p.Z); st_niels(out_niels + i, ge_to_niels_affine(fe_mul(p.X, zi), fe_mul(p.Y, zi))); }
-}
-// extended -> affine Niels (one inversion per point); used after the IPP generator fold
-__global__ void __launch_bounds__(128) k_ext_to_niels(const ge_ext *__restrict__ in, size_t n, ge_niels *__restrict__ out) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    ge_ext p = ld_ext(in + i); fe zi = fe_invert(p.Z);
-    st_niels(out + i, ge_to_niels_affine(fe_mul(p.X, zi), fe_mul(p.Y, zi)));
 }
 __global__ void __launch_bounds__(128) k_niels_to_compressed(const ge_niels *__restrict__ in, size_t n, uint8_t *__restrict__ out) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -562,12 +559,6 @@ __global__ void k_ippx_final(ippx_geom g, const sc *__restrict__ a, const sc *__
     sc_store(bytes, sc_from_mont(a[(size_t)p * g.N])); st32(out + 64 * p, bytes);
     sc_store(bytes, sc_from_mont(b[(size_t)p * g.N])); st32(out + 64 * p + 32, bytes);
 }
-// copy table entries (by index) into a contiguous device vector: G(n,m) / H(n,m) slices for the IPP prover
-__global__ void k_gather_niels(const ge_niels *__restrict__ table, const uint32_t *__restrict__ idx, uint32_t n, ge_niels *__restrict__ out) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    st_niels(out + i, ldg_niels(table + idx[i]));
-}
 
 // ------------------------------------------------------------------ range-proof batch verification kernels
 // One launch group verifies `nbatch` independent batches of `count` proofs each: every batch has its own random-linear-
@@ -743,8 +734,8 @@ __global__ void k_rp_chunk_rows(const sc *__restrict__ part_b, const uint8_t *__
     if (t < g.S) {
         sc_store(b, sc_from_mont(part_b[(size_t)ch * g.S + t]));
         if (t < 2) v = t;
-        else if (t < 2 + g.N) { uint32_t q = t - 2; v = 2 + (q / g.n) * gens_cap + (q % g.n); }
-        else { uint32_t q = t - 2 - g.N; v = 2 + gens_parties * gens_cap + (q / g.n) * gens_cap + (q % g.n); }
+        else if (t < 2 + g.N) { uint32_t q = t - 2; v = gens_slot(0u, q / g.n, q % g.n, gens_cap, gens_parties); }
+        else { uint32_t q = t - 2 - g.N; v = gens_slot(1u, q / g.n, q % g.n, gens_cap, gens_parties); }
     } else {
         uint32_t e = t - g.S, q = ch * RP_CHUNK + e / g.D;
         if (q < g.count) { ld32(b, dyn_b + ((size_t)q * g.D + e % g.D) * 32); v = BP_POINT_DYNAMIC | (dyn_base + q * g.D + e % g.D); }

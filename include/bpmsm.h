@@ -98,12 +98,10 @@ int bp_msm_indexed_batch(bp_ctx *ctx, bp_gens *gens, const uint8_t *scalars, con
 /* ---- inner-product argument, prover side, folding form ---------------------------------------- */
 /* The generator vectors G, H (and Q) live on the device for the k rounds and are folded there; the host keeps the transcript and
  * the scalar vectors a, b and calls once per round for L,R and once for the fold.  This is the form LinearProof::create
- * (linear_proof.rs:40-160) runs on; InnerProductProof::create (inner_product_proof.rs:38-193) uses the bp_ippx_* session below,
- * which keeps a and b on the device as well and never folds a point. */
+ * (linear_proof.rs:40-160) runs on, with its own G and H vectors; InnerProductProof::create (inner_product_proof.rs:38-193) uses
+ * the bp_ippx_* session below, which keeps a and b on the device as well and never folds a point. */
 typedef struct bp_ipp bp_ipp;
-/* G = bp_gens.G(n, m), H = bp_gens.H(n, m) (N = n*m points each), Q compressed */
-int bp_ipp_begin(bp_ctx *ctx, bp_gens *gens, size_t n, size_t m, const uint8_t Q[32], bp_ipp **out);
-/* arbitrary vectors: G, H = N compressed points each (the reference's Vec<RistrettoPoint> arguments) */
+/* G, H = N compressed points each (the reference's Vec<RistrettoPoint> arguments), Q compressed */
 int bp_ipp_begin_points(bp_ctx *ctx, const uint8_t *G, const uint8_t *H, size_t N, const uint8_t Q[32], bp_ipp **out);
 /* L = <sL[0..h), G_R> + <sL[h..2h), H_L> + sL[2h] Q,  R = <sR[0..h), G_L> + <sR[h..2h), H_R> + sR[2h] Q  (lines 87-113 / 153-163) */
 int bp_ipp_lr(bp_ipp *sess, size_t n_half, const uint8_t *scalars_L, const uint8_t *scalars_R, uint8_t L_out[32], uint8_t R_out[32]);

@@ -165,14 +165,6 @@ int bp_ipp_begin_points(bp_ctx *c, const uint8_t *G, const uint8_t *H, size_t N,
     if (!ok) { bp_ipp_end(s); *out = NULL; return BP_ERR_INVALID_POINT; }
     return BP_OK;
 }
-int bp_ipp_begin(bp_ctx *c, bp_gens *gens, size_t n, size_t m, const uint8_t Q[32], bp_ipp **out) {
-    if (!gens || !Q || n > gens->cap || m > gens->parties) return BP_ERR_INVALID_ARGUMENT;
-    int rc = ipp_new(c, n * m, out); if (rc) return rc;
-    bp_ipp *s = *out;
-    for (size_t q = 0; q < n * m; q++) { s->G[q] = gens->tab[2 + (q / n) * gens->cap + q % n]; s->H[q] = gens->tab[2 + gens->parties * gens->cap + (q / n) * gens->cap + q % n]; }
-    if (!ge_decode(&s->Q, Q)) { bp_ipp_end(s); *out = NULL; return BP_ERR_INVALID_POINT; }
-    return BP_OK;
-}
 int bp_ipp_lr(bp_ipp *s, size_t h, const uint8_t *sL, const uint8_t *sR, uint8_t L_out[32], uint8_t R_out[32]) {
     if (!s || !sL || !sR || !L_out || !R_out || h == 0 || 2 * h > s->N) return BP_ERR_INVALID_ARGUMENT;
     TIMED_BEGIN;
