@@ -78,6 +78,12 @@ SYMBOLS = {
 }
 
 
+# the constant-time entry points, declared in include/bpmsm_ct.h; bound on first use by ct_lib()
+CT_SYMBOLS = {
+    "bp_msm_indexed_batch_ct": (_int, [_vp, _vp, _u8p, _c.POINTER(_c.c_uint32), _c.POINTER(_c.c_uint64), _sz, _u8p, _u8p]),
+}
+
+
 class BpError(RuntimeError):
     def __init__(self, code, msg=""):
         super().__init__(f"bpmsm error {code}: {msg}")
@@ -99,6 +105,21 @@ def lib():
             fn.restype, fn.argtypes = res, args
         _lib = L
     return _lib
+
+
+_ct_bound = False
+
+
+def ct_lib():
+    """libbpmsm.so with the constant-time entry points of include/bpmsm_ct.h bound as well (AttributeError if one is missing)."""
+    global _ct_bound
+    L = lib()
+    if not _ct_bound:
+        for name, (res, args) in CT_SYMBOLS.items():
+            fn = getattr(L, name)
+            fn.restype, fn.argtypes = res, args
+        _ct_bound = True
+    return L
 
 
 HOST_LIB_PATH = os.path.join(_HERE, "libbulletproofs_host.so")
@@ -356,6 +377,30 @@ class Gens:
     @property
     def B_blinding(self):
         return self.get(3)
+
+    def msm_indexed(self, scalars: bytes, point_idx, offsets, dyn_points: bytes = b"", constant_time: bool = False):
+        """MSMs over table slots (bp_msm_indexed_batch): MSM j = sum of scalars[t] * slot point_idx[t] for t in offsets[j] .. offsets[j+1]-1;
+        slot layout: 0 = B_blinding, 1 = B, 2 + party*cap + i = G[party][i], 2 + (parties + party)*cap + i = H[party][i].
+        constant_time=True runs bp_msm_indexed_batch_ct (secret scalars; table slots only, no dyn_points).
+        Returns (status list, list of 32-byte results)."""
+        n_msm, T = len(offsets) - 1, len(point_idx)
+        idx = (ctypes.c_uint32 * max(T, 1))(*point_idx)
+        offs = (ctypes.c_uint64 * (n_msm + 1))(*offsets)
+        outs, st = ctypes.create_string_buffer(32 * max(n_msm, 1)), ctypes.create_string_buffer(max(n_msm, 1))
+        if constant_time:
+            if dyn_points:
+                raise BpError(ERR_INVALID_ARGUMENT, "the constant-time MSM takes table slots only")
+            rc = ct_lib().bp_msm_indexed_batch_ct(self.ctx._h, self._h, scalars, idx, offs, n_msm, outs, st)
+        else:
+            rc = lib().bp_msm_indexed_batch(self.ctx._h, self._h, scalars, idx, dyn_points or None, len(dyn_points) // 32, offs, n_msm, outs, st)
+        self.ctx._check(rc)
+        return list(st.raw[:n_msm]), [outs.raw[32 * i:32 * i + 32] for i in range(n_msm)]
+
+    def slot_G(self, party: int, index: int) -> int:
+        return 2 + party * self.gens_capacity + index
+
+    def slot_H(self, party: int, index: int) -> int:
+        return 2 + (self.party_capacity + party) * self.gens_capacity + index
 
     def table_export(self, d_dst: int):
         self.ctx._check(lib().bp_gens_table_export(self._h, d_dst))

@@ -25,7 +25,7 @@ def _run(cmd, cwd=None):
 
 
 def build_cuda(force=False, verbose=False):
-    srcs = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(ROOT, "include", "bpmsm.h")]
+    srcs = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(ROOT, "include", f) for f in ("bpmsm.h", "bpmsm_ct.h")]
     if not force and _newer(LIB, srcs):
         return LIB
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
@@ -42,7 +42,7 @@ def build_host(force=False):
     lib = os.path.join(ROOT, "bulletproofs_b200", "libbulletproofs_host.so")
     srcs = [os.path.join(hdir, f) for f in os.listdir(hdir)] + [os.path.join(CSRC, f) for f in ("sc.cuh", "merlin.cuh", "fe.cuh")] + [LIB]
     if force or not _newer(lib, srcs):
-        _run(["g++", "-O2", "-std=c++17", "-pthread", "-shared", "-fPIC", "-o", lib, os.path.join(hdir, "bulletproofs.cpp"), os.path.join(hdir, "r1cs.cpp"), os.path.join(hdir, "mpc.cpp"),
+        _run(["g++", "-O2", "-std=c++17", "-pthread", "-shared", "-fPIC", "-DBP_HOST_REQUIRE_CT", "-o", lib, os.path.join(hdir, "bulletproofs.cpp"), os.path.join(hdir, "r1cs.cpp"), os.path.join(hdir, "mpc.cpp"),
               "-L" + os.path.join(ROOT, "bulletproofs_b200"), "-lbpmsm", "-Wl,-rpath,$ORIGIN"])
     return lib
 

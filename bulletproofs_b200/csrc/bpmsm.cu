@@ -12,6 +12,7 @@
 #include <type_traits>
 #include <vector>
 #include "../../include/bpmsm.h"
+#include "../../include/bpmsm_ct.h"
 #include "kernels.cuh"
 
 static_assert(BP_TRANSCRIPT_BYTES == 203, "transcript wire size");
@@ -43,9 +44,11 @@ using DevBuf = Buf<false>;
 using HostBuf = Buf<true>;
 
 enum KernelId { KID_DECOMPRESS, KID_COMPRESS, KID_FROM_UNIFORM, KID_MSM_COUNT, KID_MSM_SCAN, KID_MSM_SCATTER, KID_MSM_ACCUMULATE, KID_MSM_REDUCE,
-                KID_MSM_COMBINE, KID_RP_TRANSCRIPT, KID_RP_HEAD, KID_RP_SCALARS, KID_RP_DECOMPRESS, KID_RP_STATIC_REDUCE, KID_IPP_FOLD, KID_SMALL, KID_COUNT };
+                KID_MSM_COMBINE, KID_RP_TRANSCRIPT, KID_RP_HEAD, KID_RP_SCALARS, KID_RP_DECOMPRESS, KID_RP_STATIC_REDUCE, KID_IPP_FOLD, KID_SMALL,
+                KID_MSM_CT_RECODE, KID_MSM_CT_TABLE, KID_MSM_CT_STRAUS, KID_MSM_CT_REDUCE, KID_COUNT };
 const char *const KERNEL_NAMES[KID_COUNT] = {"k_decompress", "k_compress", "k_from_uniform", "k_msm_count", "k_msm_scan", "k_msm_scatter", "k_msm_accumulate",
-                                             "k_msm_reduce", "k_msm_combine", "k_rp_transcript", "k_rp_head", "k_rp_scalars", "k_rp_decompress", "k_rp_static_reduce", "k_ipp_fold", "small_kernels"};
+                                             "k_msm_reduce", "k_msm_combine", "k_rp_transcript", "k_rp_head", "k_rp_scalars", "k_rp_decompress", "k_rp_static_reduce", "k_ipp_fold", "small_kernels",
+                                             "k_msm_ct_recode", "k_msm_ct_table", "k_msm_ct_straus", "k_msm_ct_reduce"};
 struct ProfRec { int kid; cudaEvent_t a, b; };
 
 struct VerifyState {          // what bp_rangeproof_verify_*begin leaves for *_finish
@@ -82,6 +85,7 @@ struct bp_ctx {
     // MSM scratch
     DevBuf in_scalars, in_points, in_offsets, niels, ok, msm_err, results, outs, flags, ix_pidx;
     MsmArena ar_gen;          // bp_msm*, indexed MSMs, IPP rounds, the verifier's per-proof fallback
+    DevBuf ct_digits, ct_tab, ct_chunks, ct_part;                  // constant-time indexed MSM: digits, [1..8]P tables, chunk bounds, chunk partials
     // range-proof scratch.  The inputs and verdicts stay outside rp: the kernels read their addresses from the parameter block
     // (rp.par), not from graph arguments, so they may move without invalidating the graph.
     RpGraphScratch rp;
@@ -951,6 +955,57 @@ int bp_msm_indexed_batch(bp_ctx *c, bp_gens *gens, const uint8_t *scalars, const
                 if ((point_idx[t] & BP_POINT_DYNAMIC) && !dyn_ok[point_idx[t] & 0x7fffffffu] && st[j] == BP_OK) st[j] = BP_ERR_INVALID_POINT;
     if (status) memcpy(status, st.data(), n_msm);
     return BP_OK;
+}
+
+// Constant-time form (msm_ct.cuh): table slots only.  Which kernels run, their grids and every copy follow from (T, n_msm, offsets);
+// the scalars choose nothing.  Their device copy and the digits recoded from them are cleared on the stream before the call returns.
+int bp_msm_indexed_batch_ct(bp_ctx *c, bp_gens *gens, const uint8_t *scalars, const uint32_t *point_idx, const uint64_t *offsets, size_t n_msm,
+                            uint8_t *outs, uint8_t *status) {
+    if (!c || !offsets || !outs || n_msm == 0) return BP_ERR_INVALID_ARGUMENT;
+    size_t T = offsets[n_msm];
+    if (offsets[0] != 0 || T == 0 || T >= (1u << 31) || !scalars || !point_idx) return BP_ERR_INVALID_ARGUMENT;
+    BUSY_CHECK(c);
+    CK(c, cudaSetDevice(c->device));
+    if (!gens) return BP_ERR_INVALID_ARGUMENT;
+    for (size_t t = 0; t < T; t++) if (point_idx[t] >= gens->n_points) return BP_ERR_INVALID_ARGUMENT;      // dynamic points are not accepted
+    std::vector<uint32_t> off32(n_msm + 1);
+    for (size_t j = 0; j <= n_msm; j++) { if (j && offsets[j] < offsets[j - 1]) return BP_ERR_LENGTH_MISMATCH; off32[j] = (uint32_t)offsets[j]; }
+    // chunks of at most `ch` consecutive terms, never across an MSM boundary; ch grows while the grid would still hold >= 148 x 128 threads,
+    // trading parallelism for fewer doublings per term (four per window per chunk)
+    uint32_t ch = 1;
+    while (ch < 16 && T / (2 * ch) >= 148 * 128) ch *= 2;
+    std::vector<uint32_t> bounds;            // [chunk starts (n_chunks) | T | first chunk of each MSM (n_msm + 1)]
+    std::vector<uint32_t> msm_first(n_msm + 1);
+    for (size_t j = 0; j < n_msm; j++) {
+        msm_first[j] = (uint32_t)bounds.size();
+        for (uint32_t t = off32[j]; t < off32[j + 1]; t += ch) bounds.push_back(t);
+    }
+    const uint32_t n_chunks = (uint32_t)bounds.size(); msm_first[n_msm] = n_chunks;
+    bounds.push_back((uint32_t)T);
+    bounds.insert(bounds.end(), msm_first.begin(), msm_first.end());
+    cudaStream_t s = c->stream;
+    const uint32_t M = (uint32_t)n_msm;
+    CK(c, c->in_scalars.ensure(T * 32)); CK(c, c->in_offsets.ensure((n_msm + 1) * 4)); CK(c, c->ix_pidx.ensure(T * 4));
+    CK(c, c->outs.ensure(n_msm * 32)); CK(c, c->flags.ensure(n_msm)); CK(c, c->msm_err.ensure((size_t)M * 4)); CK(c, c->results.ensure((size_t)M * sizeof(ge_ext)));
+    CK(c, c->ct_digits.ensure(T * CT_DIGITS)); CK(c, c->ct_tab.ensure(T * CT_TABLE * sizeof(ge_ext)));
+    CK(c, c->ct_chunks.ensure(bounds.size() * 4)); CK(c, c->ct_part.ensure((size_t)n_chunks * sizeof(ge_ext)));
+    CK(c, cudaMemcpyAsync(c->in_scalars.p, scalars, T * 32, cudaMemcpyHostToDevice, s));
+    CK(c, cudaMemcpyAsync(c->in_offsets.p, off32.data(), (n_msm + 1) * 4, cudaMemcpyHostToDevice, s));
+    CK(c, cudaMemcpyAsync(c->ix_pidx.p, point_idx, T * 4, cudaMemcpyHostToDevice, s));
+    CK(c, cudaMemcpyAsync(c->ct_chunks.p, bounds.data(), bounds.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(c, cudaMemsetAsync(c->msm_err.p, 0, (size_t)M * 4, s));
+    const uint32_t *d_chunks = c->ct_chunks.as<uint32_t>(), *d_msm_first = d_chunks + n_chunks + 1;
+    LAUNCH(c, KID_MSM_CT_RECODE, k_msm_ct_recode<<<blocks_for(T, 128), 128, 0, s>>>(c->in_scalars.as<uint8_t>(), c->in_offsets.as<uint32_t>(), M, (uint32_t)T,
+                                                                                    c->ct_digits.as<int8_t>(), c->msm_err.as<uint32_t>()));
+    LAUNCH(c, KID_MSM_CT_TABLE, k_msm_ct_table<<<blocks_for(T, 128), 128, 0, s>>>(c->ix_pidx.as<uint32_t>(), (uint32_t)T, gens->d_table(), c->ct_tab.as<ge_ext>()));
+    LAUNCH(c, KID_MSM_CT_STRAUS, k_msm_ct_straus<<<blocks_for(n_chunks, 128), 128, 0, s>>>(d_chunks, n_chunks, c->ct_digits.as<int8_t>(), c->ct_tab.as<ge_ext>(), c->ct_part.as<ge_ext>()));
+    LAUNCH(c, KID_MSM_CT_REDUCE, k_msm_ct_reduce<<<M, CT_REDUCE_THREADS, 0, s>>>(c->ct_part.as<ge_ext>(), d_msm_first, c->results.as<ge_ext>()));
+    LAUNCH(c, KID_COMPRESS, k_compress<<<blocks_for(M, 128), 128, 0, s>>>(c->results.as<ge_ext>(), M, c->outs.as<uint8_t>()));
+    LAUNCH(c, KID_SMALL, k_msm_status<<<blocks_for(M, 128), 128, 0, s>>>(c->msm_err.as<uint32_t>(), M, c->flags.as<uint8_t>()));
+    // clear_on_drop of the reference's secrets: the scalars and their digits do not outlive the call on the device
+    CK(c, cudaMemsetAsync(c->in_scalars.p, 0, T * 32, s));
+    CK(c, cudaMemsetAsync(c->ct_digits.p, 0, T * CT_DIGITS, s));
+    return msm_copy_out(c, n_msm, outs, status);
 }
 
 int bp_ipp_begin_points(bp_ctx *c, const uint8_t *G, const uint8_t *H, size_t N, const uint8_t Q[32], bp_ipp **out) {

@@ -434,6 +434,9 @@ BP_HD bool fe_is_zero(const fe &a) { fe c = fe_canon(a); uint32_t z = 0; for (in
 BP_HD bool fe_eq(const fe &a, const fe &b) { return fe_is_zero(fe_sub(a, b)); }
 BP_HD fe fe_select(const fe &a, const fe &b, bool pick_b) { fe r; uint32_t m = 0u - (uint32_t)pick_b; for (int i = 0; i < 8; i++) r.v[i] = (b.v[i] & m) | (a.v[i] & ~m); return r; }
 BP_HD fe fe_cneg(const fe &a, bool neg) { return fe_select(a, fe_neg(a), neg); }
+// mask-taking forms for secret conditions (msm_ct.cuh): mask is all-ones or zero and is never turned into a bool
+BP_HD fe fe_select_mask(const fe &a, const fe &b, uint32_t mask) { fe r; for (int i = 0; i < 8; i++) r.v[i] = a.v[i] ^ ((a.v[i] ^ b.v[i]) & mask); return r; }
+BP_HD fe fe_cneg_mask(const fe &a, uint32_t mask) { return fe_select_mask(a, fe_neg(a), mask); }
 BP_HD fe fe_abs(const fe &a) { return fe_cneg(a, fe_is_negative(a)); }
 
 // z^(2^250-1) with z^11 on the side: the shared ladder of invert and pow22523

@@ -9,6 +9,7 @@
 #include "merlin.cuh"
 #include "rp.cuh"
 #include "msm_common.cuh"
+#include "msm_ct.cuh"
 
 #define BP_POINT_DYNAMIC 0x80000000u     // point_idx flag: index into the per-call (dynamic) point array
 
@@ -793,4 +794,81 @@ __global__ void k_rp_verdict_proofs(const uint32_t *__restrict__ status, const u
     if (p >= count) return;
     uint32_t st = rp_eff_status(status[p], dec_bad[p]);
     verdict[p] = st != BP_PROOF_OK ? st : (ge_is_identity(ld_ext(results + p)) ? (uint32_t)BP_PROOF_OK : (uint32_t)BP_PROOF_VERIFICATION_ERROR);
+}
+
+// ------------------------------------------------------------------ constant-time indexed MSM (msm_ct.cuh, bp_msm_indexed_batch_ct)
+// recode: one thread per term.  digits: T x 64 signed bytes; msm_err bit 1 = a non-canonical scalar in that MSM (the atomic is issued
+// for every term, with the flag as its operand, so neither its address nor its presence depends on the scalar)
+__global__ void __launch_bounds__(128) k_msm_ct_recode(const uint8_t *__restrict__ scalars, const uint32_t *__restrict__ offsets, uint32_t n_msm, uint32_t T,
+                                                       int8_t *__restrict__ digits, uint32_t *__restrict__ msm_err) {
+    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= T) return;
+    const uint4 *p = reinterpret_cast<const uint4 *>(scalars + 32 * (size_t)t);
+    uint4 a = p[0], b = p[1];
+    uint32_t s[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+    uint32_t bad = ct_scalar_geq_l_mask(s);
+    for (int i = 0; i < 8; i++) s[i] &= ~bad;                        // a rejected scalar contributes nothing
+    uint32_t d[CT_DIGITS];
+    ct_recode_radix16(s, d);
+    uint32_t w[CT_DIGITS / 4];
+#pragma unroll
+    for (int i = 0; i < CT_DIGITS / 4; i++) w[i] = (d[4 * i] & 0xffu) | ((d[4 * i + 1] & 0xffu) << 8) | ((d[4 * i + 2] & 0xffu) << 16) | ((d[4 * i + 3] & 0xffu) << 24);
+    uint4 *o = reinterpret_cast<uint4 *>(digits + (size_t)CT_DIGITS * t);
+#pragma unroll
+    for (int i = 0; i < CT_DIGITS / 16; i++) o[i] = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
+    uint32_t msm = n_msm == 1 ? 0u : msm_of_term(offsets, n_msm, t);
+    atomicOr(msm_err + msm, bad & 2u);
+}
+
+// table: one thread per term, [1..8]P of table slot point_idx[t] (public data only)
+__global__ void __launch_bounds__(128) k_msm_ct_table(const uint32_t *__restrict__ point_idx, uint32_t T, const ge_niels *__restrict__ gens, ge_ext *__restrict__ tab) {
+    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= T) return;
+    ge_ext *o = tab + (size_t)CT_TABLE * t;
+    ct_table(ge_from_niels(ldg_niels(gens + __ldg(point_idx + t))), [&](int j, const ge_ext &p) { st_ext(o + j, p); });
+}
+
+// straus: one thread per chunk [chunks[c], chunks[c+1]) of consecutive terms of one MSM
+__global__ void __launch_bounds__(128) k_msm_ct_straus(const uint32_t *__restrict__ chunks, uint32_t n_chunks, const int8_t *__restrict__ digits,
+                                                       const ge_ext *__restrict__ tab, ge_ext *__restrict__ partial) {
+    uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n_chunks) return;
+    const uint32_t lo = __ldg(chunks + c), hi = __ldg(chunks + c + 1);
+    ge_ext acc = ge_identity();
+#pragma unroll 1
+    for (int w = CT_DIGITS - 1; w >= 0; w--) {
+        if (w != CT_DIGITS - 1) {
+#pragma unroll 1
+            for (int i = 0; i < 4; i++) acc = ge_dbl(acc);
+        }
+#pragma unroll 1
+        for (uint32_t t = lo; t < hi; t++) {
+            const uint32_t d = (uint32_t)(int32_t)__ldg(digits + (size_t)CT_DIGITS * t + w);
+            const uint32_t *base = reinterpret_cast<const uint32_t *>(tab + (size_t)CT_TABLE * t);
+            ge_ext e = ct_lookup(d, [&](uint32_t j, int k, uint32_t *v) { uint4 x = __ldg(reinterpret_cast<const uint4 *>(base + 32 * j + k)); v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w; });
+            acc = ge_add(acc, e);
+        }
+    }
+    st_ext(partial + c, acc);
+}
+
+// reduce: one block per MSM; thread i adds chunks i, i + blockDim, ... of the MSM, then a shuffle tree and one shared-memory round
+#define CT_REDUCE_THREADS 128
+__global__ void __launch_bounds__(CT_REDUCE_THREADS) k_msm_ct_reduce(const ge_ext *__restrict__ partial, const uint32_t *__restrict__ msm_chunks, ge_ext *__restrict__ results) {
+    __shared__ ge_ext sm[CT_REDUCE_THREADS / 32];
+    const uint32_t m = blockIdx.x, lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const uint32_t c0 = __ldg(msm_chunks + m), c1 = __ldg(msm_chunks + m + 1);
+    ge_ext acc = ge_identity();
+#pragma unroll 1
+    for (uint32_t c = c0 + threadIdx.x; c < c1; c += blockDim.x) acc = ge_add(acc, ld_ext(partial + c));
+#pragma unroll 1
+    for (int d = 16; d >= 1; d >>= 1) { ge_ext o = shfl_down_ext(acc, d); acc = ge_add(acc, o); }
+    if (lane == 0) sm[wid] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        ge_ext r = sm[0];
+#pragma unroll 1
+        for (uint32_t k = 1; k < CT_REDUCE_THREADS / 32; k++) r = ge_add(r, sm[k]);
+        st_ext(results + m, r);
+    }
 }

@@ -307,7 +307,12 @@ struct ProverState {
 };
 // the MSMs one proof asks for in a phase (scalars, table slots, end offsets), built per proof in parallel and merged into one device call
 struct MsmReq { std::vector<Scalar> sc; std::vector<uint32_t> idx; std::vector<uint64_t> off; };
-bool run_requests(Device &dev, const BulletproofGens &gens, const std::vector<MsmReq> &reqs, std::vector<ProverState> &st, std::vector<uint8_t> &out) {
+// the two indexed-MSM entry points with one signature: constant-time for secret scalars (phases 1-2), variable-time for Q = w B (phase 3)
+using IndexedMsm = int (*)(bp_ctx *, bp_gens *, const uint8_t *, const uint32_t *, const uint64_t *, size_t, uint8_t *, uint8_t *);
+int indexed_msm_vartime(bp_ctx *c, bp_gens *g, const uint8_t *sc, const uint32_t *idx, const uint64_t *off, size_t n_msm, uint8_t *out, uint8_t *st) {
+    return bp_msm_indexed_batch(c, g, sc, idx, nullptr, 0, off, n_msm, out, st);
+}
+bool run_requests(Device &dev, const BulletproofGens &gens, IndexedMsm msm, const std::vector<MsmReq> &reqs, std::vector<ProverState> &st, std::vector<uint8_t> &out) {
     size_t terms = 0, n_msm = 0;
     for (const MsmReq &r : reqs) { terms += r.sc.size(); n_msm += r.off.size(); }
     if (n_msm == 0) return false;
@@ -318,7 +323,7 @@ bool run_requests(Device &dev, const BulletproofGens &gens, const std::vector<Ms
         for (size_t i = 0; i < reqs[p].sc.size(); i++) { reqs[p].sc[i].write(sc.data() + 32 * (base[p] + i)); idx[base[p] + i] = reqs[p].idx[i]; }
     });
     out.assign(32 * n_msm, 0); std::vector<uint8_t> stt(n_msm);
-    check(bp_msm_indexed_batch(dev.ctx, gens.handle, sc.data(), idx.data(), nullptr, 0, off.data(), n_msm, out.data(), stt.data()), dev.ctx, "bp_msm_indexed_batch");
+    check(msm(dev.ctx, gens.handle, sc.data(), idx.data(), off.data(), n_msm, out.data(), stt.data()), dev.ctx, "indexed MSM");
     return true;
 }
 }  // namespace
@@ -329,7 +334,7 @@ bool run_requests(Device &dev, const BulletproofGens &gens, const std::vector<Ms
 void RangeProof::prove_many(Device &dev, const BulletproofGens &gens, size_t n, std::vector<RangeProofJob> &jobs) {
     const size_t B = jobs.size();
     std::vector<ProverState> st(B);
-    const Scalar one = Scalar::one(), minus_one = -one;
+    const Scalar one = Scalar::one();
     // ---- phase 1: parameter checks, RNG draws, bit commitments
     {
         std::vector<MsmReq> reqs(B);
@@ -351,11 +356,12 @@ void RangeProof::prove_many(Device &dev, const BulletproofGens &gens, size_t n, 
                 for (size_t i = 0; i < n; i++) S.sR[j * n + i] = Scalar::random(*J.rng);
             }
             // m + 2 constant-base MSMs: V_j = v_j B + v~_j B~ (party.rs:51), A = sum_j (a~_j B~ + sum_i [bit ? G : -H]) (party.rs:100-112,
-            // dealer.rs:112-113), S = sum_j (s~_j B~ + <s_L, G_j> + <s_R, H_j>) (party.rs:119-124, dealer.rs:115-116)
+            // dealer.rs:112-113), S = sum_j (s~_j B~ + <s_L, G_j> + <s_R, H_j>) (party.rs:119-124, dealer.rs:115-116).  A is written with
+            // every G_i and H_i present, sum_i (b_i G_i + (b_i - 1) H_i): the same point, with point indices that do not depend on the bits.
             for (size_t j = 0; j < m; j++) { sc.push_back(Scalar::from_u64(J.values[j])); idx.push_back(gens.slot_B()); sc.push_back(J.blindings[j]); idx.push_back(gens.slot_B_blinding()); off.push_back(sc.size()); }
             for (size_t j = 0; j < m; j++) {
                 sc.push_back(S.a_bl[j]); idx.push_back(gens.slot_B_blinding());
-                for (size_t i = 0; i < n; i++) { bool bit = (J.values[j] >> i) & 1; sc.push_back(bit ? one : minus_one); idx.push_back(bit ? gens.slot_G(j, i) : gens.slot_H(j, i)); }
+                for (size_t i = 0; i < n; i++) { Scalar b = Scalar::from_u64((J.values[j] >> i) & 1); sc.push_back(b); idx.push_back(gens.slot_G(j, i)); sc.push_back(b - one); idx.push_back(gens.slot_H(j, i)); }
             }
             off.push_back(sc.size());
             for (size_t j = 0; j < m; j++) {
@@ -366,7 +372,7 @@ void RangeProof::prove_many(Device &dev, const BulletproofGens &gens, size_t n, 
             off.push_back(sc.size());
         });
         std::vector<uint8_t> out;
-        if (!run_requests(dev, gens, reqs, st, out)) return;
+        if (!run_requests(dev, gens, secret_indexed_msm, reqs, st, out)) return;
         for (size_t p = 0; p < B; p++) {
             if (!st[p].live) continue;
             RangeProofJob &J = jobs[p]; size_t m = st[p].m; const uint8_t *o = out.data() + 32 * st[p].out_base;
@@ -411,7 +417,7 @@ void RangeProof::prove_many(Device &dev, const BulletproofGens &gens, size_t n, 
             off.push_back(sc.size());
         });
         std::vector<uint8_t> out;
-        if (!run_requests(dev, gens, reqs, st, out)) return;
+        if (!run_requests(dev, gens, secret_indexed_msm, reqs, st, out)) return;
         for (size_t p = 0; p < B; p++) {
             if (!st[p].live) continue;
             memcpy(jobs[p].proof.T_1.data(), out.data() + 32 * st[p].out_base, 32); memcpy(jobs[p].proof.T_2.data(), out.data() + 32 * (st[p].out_base + 1), 32);
@@ -444,7 +450,7 @@ void RangeProof::prove_many(Device &dev, const BulletproofGens &gens, size_t n, 
             for (size_t i = 0; i < N; i++) { S.Hf[i] = e; e *= y_inv; }                                   // dealer.rs:258-261
         });
         std::vector<uint8_t> out;
-        if (!run_requests(dev, gens, reqs, st, out)) return;
+        if (!run_requests(dev, gens, indexed_msm_vartime, reqs, st, out)) return;          // w is a public challenge (dealer.rs:256)
         for (size_t p = 0; p < B; p++) if (st[p].live) memcpy(st[p].Q.data(), out.data() + 32 * st[p].out_base, 32);
     }
     // ---- phase 4: the inner-product arguments, grouped by aggregation size (one device session per distinct m)

@@ -21,6 +21,7 @@
 #include <string>
 #include <vector>
 #include "../../include/bpmsm.h"
+#include "../../include/bpmsm_ct.h"
 #include "../csrc/merlin.cuh"
 #include "../csrc/sc.cuh"
 
@@ -111,6 +112,22 @@ public:
 };
 
 // one device + stream (bp_ctx)
+// The MSM of every commitment to a secret (PedersenGens::commit, A, S, T_i; the R1CS A_I, A_O, S): bp_msm_indexed_batch_ct, which is
+// constant-time in the scalars (DESIGN.md "constant-time policy").  The library build (bulletproofs_b200/build.py) defines
+// BP_HOST_REQUIRE_CT: the call is then a plain reference, resolved when the library loads, and there is no other path.  Without the
+// define the reference is weak, so that the mirror also links against an engine that predates the entry point -- the CPU test
+// harness's stand-in on the oracle's arithmetic, which makes no timing claim -- and such an engine computes the same group elements
+// with bp_msm_indexed_batch.
+#ifndef BP_HOST_REQUIRE_CT
+#pragma weak bp_msm_indexed_batch_ct
+#endif
+static inline int secret_indexed_msm(bp_ctx *c, bp_gens *g, const uint8_t *sc, const uint32_t *idx, const uint64_t *off, size_t n_msm, uint8_t *out, uint8_t *st) {
+#ifndef BP_HOST_REQUIRE_CT
+    if (!bp_msm_indexed_batch_ct) return bp_msm_indexed_batch(c, g, sc, idx, nullptr, 0, off, n_msm, out, st);
+#endif
+    return bp_msm_indexed_batch_ct(c, g, sc, idx, off, n_msm, out, st);
+}
+
 class Device {
 public:
     bp_ctx *ctx;

@@ -85,7 +85,7 @@ MPCError Party::new_(Device &dev, const BulletproofGens &gens, uint64_t v, const
     if (gens.gens_capacity < n) return MPCError::InvalidGeneratorsLength;
     std::vector<Scalar> sc = {Scalar::from_u64(v), v_blinding}; uint32_t idx[2] = {gens.slot_B(), gens.slot_B_blinding()}; uint64_t offs[2] = {0, 2}; uint8_t st;
     out = PartyAwaitingPosition{&dev, &gens, n, v, v_blinding, {}};
-    check(bp_msm_indexed_batch(dev.ctx, gens.handle, pack(sc).data(), idx, nullptr, 0, offs, 1, out.V.data(), &st), dev.ctx, "bp_msm_indexed_batch");     // pc_gens.commit :50
+    check(secret_indexed_msm(dev.ctx, gens.handle, pack(sc).data(), idx, offs, 1, out.V.data(), &st), dev.ctx, "secret_indexed_msm");     // pc_gens.commit :50
     return MPCError::Ok;
 }
 MPCError PartyAwaitingPosition::assign_position_with_rng(size_t j, Rng &rng, PartyAwaitingBitChallenge &next, BitCommitment &out) const {
@@ -95,16 +95,17 @@ MPCError PartyAwaitingPosition::assign_position_with_rng(size_t j, Rng &rng, Par
     next.s_L.resize(n); next.s_R.resize(n);
     for (size_t i = 0; i < n; i++) next.s_L[i] = Scalar::random(rng);                                       // :115
     for (size_t i = 0; i < n; i++) next.s_R[i] = Scalar::random(rng);                                       // :116
-    // A_j = a~ B~ + sum_i (bit ? G_i : -H_i)  (:100-112);  S_j = s~ B~ + <s_L, G> + <s_R, H>  (:119-124): two MSMs, one call
-    std::vector<Scalar> sc; std::vector<uint32_t> idx; Scalar one = Scalar::one(), minus_one = -one;
+    // A_j = a~ B~ + sum_i (bit ? G_i : -H_i)  (:100-112), written as a~ B~ + sum_i (b_i G_i + (b_i - 1) H_i) so that the point indices do
+    // not depend on the bits;  S_j = s~ B~ + <s_L, G> + <s_R, H>  (:119-124): two constant-time MSMs, one call
+    std::vector<Scalar> sc; std::vector<uint32_t> idx; Scalar one = Scalar::one();
     sc.push_back(next.a_blinding); idx.push_back(gens->slot_B_blinding());
-    for (size_t i = 0; i < n; i++) { bool bit = (v >> i) & 1; sc.push_back(bit ? one : minus_one); idx.push_back(bit ? gens->slot_G(j, i) : gens->slot_H(j, i)); }
+    for (size_t i = 0; i < n; i++) { Scalar b = Scalar::from_u64((v >> i) & 1); sc.push_back(b); idx.push_back(gens->slot_G(j, i)); sc.push_back(b - one); idx.push_back(gens->slot_H(j, i)); }
     size_t split = sc.size();
     sc.push_back(next.s_blinding); idx.push_back(gens->slot_B_blinding());
     for (size_t i = 0; i < n; i++) { sc.push_back(next.s_L[i]); idx.push_back(gens->slot_G(j, i)); }
     for (size_t i = 0; i < n; i++) { sc.push_back(next.s_R[i]); idx.push_back(gens->slot_H(j, i)); }
     uint64_t offs[3] = {0, split, sc.size()}; uint8_t outs[64], st[2];
-    check(bp_msm_indexed_batch(dev->ctx, gens->handle, pack(sc).data(), idx.data(), nullptr, 0, offs, 2, outs, st), dev->ctx, "bp_msm_indexed_batch");
+    check(secret_indexed_msm(dev->ctx, gens->handle, pack(sc).data(), idx.data(), offs, 2, outs, st), dev->ctx, "secret_indexed_msm");
     out.V_j = V; memcpy(out.A_j.data(), outs, 32); memcpy(out.S_j.data(), outs + 32, 32);
     return MPCError::Ok;
 }
@@ -128,7 +129,7 @@ void PartyAwaitingBitChallenge::apply_challenge_with_rng(const BitChallenge &vc,
     next.v_blinding = v_blinding; next.a_blinding = a_blinding; next.s_blinding = s_blinding;
     std::vector<Scalar> sc = {next.t1, next.t_1_blinding, next.t2, next.t_2_blinding};                      // T_1_j, T_2_j :216-217
     uint32_t idx[4] = {gens->slot_B(), gens->slot_B_blinding(), gens->slot_B(), gens->slot_B_blinding()}; uint64_t offs[3] = {0, 2, 4}; uint8_t outs[64], st[2];
-    check(bp_msm_indexed_batch(dev->ctx, gens->handle, pack(sc).data(), idx, nullptr, 0, offs, 2, outs, st), dev->ctx, "bp_msm_indexed_batch");
+    check(secret_indexed_msm(dev->ctx, gens->handle, pack(sc).data(), idx, offs, 2, outs, st), dev->ctx, "secret_indexed_msm");
     memcpy(out.T_1_j.data(), outs, 32); memcpy(out.T_2_j.data(), outs + 32, 32);
 }
 MPCError PartyAwaitingPolyChallenge::apply_challenge(const PolyChallenge &pc, ProofShare &out) const {

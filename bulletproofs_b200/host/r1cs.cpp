@@ -92,7 +92,7 @@ std::pair<CompressedRistretto, Variable> Prover::commit(const Scalar &v, const S
     // PedersenGens::commit (generators.rs:39-41) on the GPU
     std::vector<Scalar> sc = {v, v_blinding}; uint32_t idx[2] = {gens_.slot_B(), gens_.slot_B_blinding()}; uint64_t off[2] = {0, 2}; uint8_t st;
     CompressedRistretto V;
-    check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, pack(sc).data(), idx, nullptr, 0, off, 1, V.data(), &st), dev_.ctx, "commit");
+    check(secret_indexed_msm(dev_.ctx, gens_.handle, pack(sc).data(), idx, off, 1, V.data(), &st), dev_.ctx, "commit");
     t_.append_point("V", V);
     return {V, Variable{VarKind::Committed, i}};
 }
@@ -104,7 +104,7 @@ std::vector<std::pair<CompressedRistretto, Variable>> Prover::commit_vec(const s
     std::vector<Scalar> sc(2 * m); std::vector<uint32_t> idx(2 * m); std::vector<uint64_t> off(m + 1); std::vector<uint8_t> outs(32 * m), st(m);
     for (size_t i = 0; i < m; i++) { sc[2 * i] = v[i]; sc[2 * i + 1] = v_blinding[i]; idx[2 * i] = gens_.slot_B(); idx[2 * i + 1] = gens_.slot_B_blinding(); off[i] = 2 * i; }
     off[m] = 2 * m;
-    check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), nullptr, 0, off.data(), m, outs.data(), st.data()), dev_.ctx, "commit_vec");
+    check(secret_indexed_msm(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), off.data(), m, outs.data(), st.data()), dev_.ctx, "commit_vec");
     for (size_t i = 0; i < m; i++) {
         size_t j = v_.size(); v_.push_back(v[i]); v_blinding_.push_back(v_blinding[i]);
         memcpy(out[i].first.data(), outs.data() + 32 * i, 32); out[i].second = Variable{VarKind::Committed, j};
@@ -176,7 +176,7 @@ R1CSError Prover::prove(Rng &external_rng, R1CSProof &proof) {
         push_vector_commitment(sc, idx, off, gens_, o_bl1, a_O_.data(), nullptr, 0, n1);
         push_vector_commitment(sc, idx, off, gens_, s_bl1, s_L.data(), s_R.data(), 0, n1);
         uint8_t out[96], st[3];
-        check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), nullptr, 0, off.data(), 3, out, st), dev_.ctx, "phase-1 commitments");
+        check(secret_indexed_msm(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), off.data(), 3, out, st), dev_.ctx, "phase-1 commitments");
         memcpy(proof.A_I1.data(), out, 32); memcpy(proof.A_O1.data(), out + 32, 32); memcpy(proof.S1.data(), out + 64, 32);
     }
     t_.append_point("A_I1", proof.A_I1); t_.append_point("A_O1", proof.A_O1); t_.append_point("S1", proof.S1);
@@ -202,7 +202,7 @@ R1CSError Prover::prove(Rng &external_rng, R1CSProof &proof) {
         push_vector_commitment(sc, idx, off, gens_, o_bl2, a_O_.data() + n1, nullptr, n1, n2);
         push_vector_commitment(sc, idx, off, gens_, s_bl2, s_L.data() + n1, s_R.data() + n1, n1, n2);
         uint8_t out[96], st[3];
-        check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), nullptr, 0, off.data(), 3, out, st), dev_.ctx, "phase-2 commitments");
+        check(secret_indexed_msm(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), off.data(), 3, out, st), dev_.ctx, "phase-2 commitments");
         memcpy(proof.A_I2.data(), out, 32); memcpy(proof.A_O2.data(), out + 32, 32); memcpy(proof.S2.data(), out + 64, 32);
     }
     t_.append_point("A_I2", proof.A_I2); t_.append_point("A_O2", proof.A_O2); t_.append_point("S2", proof.S2);
@@ -232,7 +232,7 @@ R1CSError Prover::prove(Rng &external_rng, R1CSProof &proof) {
         std::vector<Scalar> sc = {t1, t1b, t3, t3b, t4, t4b, t5, t5b, t6, t6b}; std::vector<uint32_t> idx; std::vector<uint64_t> off = {0};
         for (int k = 0; k < 5; k++) { idx.push_back(gens_.slot_B()); idx.push_back(gens_.slot_B_blinding()); off.push_back(2 * (k + 1)); }
         uint8_t out[160], st[5];
-        check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), nullptr, 0, off.data(), 5, out, st), dev_.ctx, "T commitments");
+        check(secret_indexed_msm(dev_.ctx, gens_.handle, pack(sc).data(), idx.data(), off.data(), 5, out, st), dev_.ctx, "T commitments");
         CompressedRistretto *Ts[5] = {&proof.T_1, &proof.T_3, &proof.T_4, &proof.T_5, &proof.T_6};
         for (int k = 0; k < 5; k++) memcpy(Ts[k]->data(), out + 32 * k, 32);
     }
@@ -255,7 +255,7 @@ R1CSError Prover::prove(Rng &external_rng, R1CSProof &proof) {
     t_.append_scalar("t_x", proof.t_x); t_.append_scalar("t_x_blinding", proof.t_x_blinding); t_.append_scalar("e_blinding", proof.e_blinding);
     Scalar w = t_.challenge_scalar("w");
     CompressedRistretto Q; uint32_t qi = gens_.slot_B(); uint64_t qo[2] = {0, 1}; uint8_t qs;
-    check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, w.to_bytes().data(), &qi, nullptr, 0, qo, 1, Q.data(), &qs), dev_.ctx, "Q");
+    check(bp_msm_indexed_batch(dev_.ctx, gens_.handle, w.to_bytes().data(), &qi, nullptr, 0, qo, 1, Q.data(), &qs), dev_.ctx, "Q");     // w is a public challenge: variable-time
     std::vector<Scalar> Gf(padded_n), Hf(padded_n);
     parallel_for(nch, [&](size_t c) {                                                                                 // prover.rs:648-656
         for (size_t i = c * CH; i < std::min(padded_n, (c + 1) * CH); i++) { Gf[i] = i < n1 ? Scalar::one() : u; Hf[i] = exp_y_inv[i] * Gf[i]; }

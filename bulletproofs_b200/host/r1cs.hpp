@@ -4,8 +4,9 @@
 //   Prover::{new, commit, prove}           /root/reference/src/r1cs/prover.rs:242-698
 //   Verifier::{new, commit, verify}        /root/reference/src/r1cs/verifier.rs:204-500
 //   R1CSProof::{to_bytes, from_bytes}      /root/reference/src/r1cs/proof.rs:71-204
-// Every multiscalar multiplication (A_I/A_O/S in both phases, the T commitments, Q, the IPP rounds,
-// the verifier's mega-check) runs on the GPU through bp_msm_indexed_batch / bp_ipp_*.
+// Every multiscalar multiplication runs on the GPU: the commitments to secrets (commit, A_I/A_O/S in both phases, the
+// T commitments) through the constant-time bp_msm_indexed_batch_ct; Q, the IPP rounds and the verifier's mega-check through
+// the variable-time bp_msm_indexed_batch / bp_ippx_*, as the reference does.
 #pragma once
 #include <functional>
 #include <memory>

@@ -15,9 +15,12 @@
  * Threading: a bp_ctx is one device + one CUDA stream and is not thread-safe; different
  * contexts may be used concurrently.  There is no hidden global state and no CPU fallback:
  * every call fails with BP_ERR_CUDA when no sm_100 device is usable.
- * Timing: all work is variable-time (like the reference's vartime_* calls).  The reference's
- * constant-time `multiscalar_mul` sites (prover secrets) are served by the same variable-time
- * kernels; see DESIGN.md "constant-time policy".
+ * Timing: bp_msm_indexed_batch_ct (include/bpmsm_ct.h) is constant-time in its scalars: which kernels run, their grids, every memory address and every
+ * copy depend only on the term count, the offsets and the point indices, and the only scalar-derived value it returns besides the
+ * results is the per-MSM canonicality status.  Its point indices, offsets and results are public.  Every other entry point is
+ * variable-time in all of its inputs, like the reference's vartime_* calls: use them for public data (verification, challenges)
+ * only.  The C++ host mirror routes the reference's constant-time `multiscalar_mul` sites through the ct entry point; see
+ * DESIGN.md "constant-time policy" for what is and is not covered.
  */
 #ifndef BPMSM_H
 #define BPMSM_H
@@ -73,7 +76,7 @@ int bp_from_uniform_bytes_batch(bp_ctx *ctx, const uint8_t *uniform, size_t n, u
 /* RistrettoPoint::vartime_multiscalar_mul / optional_multiscalar_mul on wire types:
  *   out = compress( sum_i scalars[i] * decompress(points[i]) ).
  * Call sites replaced: inner_product_proof.rs:87,101,127,131,153,159,177,178,308;
- * range_proof/mod.rs:421; range_proof/messages.rs:128,149; generators.rs:40; range_proof/party.rs:119.
+ * range_proof/mod.rs:421; range_proof/messages.rs:128,149.
  * Returns BP_ERR_INVALID_POINT if any point does not decode (the reference's `None`). */
 int bp_msm(bp_ctx *ctx, const uint8_t *scalars, const uint8_t *points, size_t n, uint8_t out[32]);
 /* n_msm independent MSMs in one launch sequence: MSM j uses terms offsets[j] .. offsets[j+1]-1.
@@ -88,9 +91,9 @@ int bp_msm_batch_device(bp_ctx *ctx, const void *d_scalars, const void *d_points
 /* MSMs whose points are generator-table entries and/or caller-supplied compressed points:
  * point_idx[t] < 2^31 selects table slot point_idx[t] of `gens` (layout of bp_gens_device_table: 0 = B_blinding,
  * 1 = B, 2 + party*cap + i = G[party][i], 2 + parties*cap + party*cap + i = H[party][i]); point_idx[t] = 2^31 | j
- * selects dyn_points[j].  This is how the prover-side constant-base call sites run without re-uploading the table:
- * PedersenGens::commit (generators.rs:39-41), A and S (range_proof/party.rs:100-124), T_1/T_2 (party.rs:216-217),
- * Q = w*B (dealer.rs:256), and the stand-alone IPP verification MSM (inner_product_proof.rs:308-319). */
+ * selects dyn_points[j].  This is how the public-scalar constant-base call sites run without re-uploading the table: Q = w*B
+ * (dealer.rs:256), ProofShare::audit_share (messages.rs:128,149) and the R1CS verifier's mega-check.  The prover's commitments to
+ * secrets (PedersenGens::commit, A, S, T_1/T_2) use bp_msm_indexed_batch_ct (include/bpmsm_ct.h). */
 int bp_msm_indexed_batch(bp_ctx *ctx, bp_gens *gens, const uint8_t *scalars, const uint32_t *point_idx,
                          const uint8_t *dyn_points, size_t n_dyn, const uint64_t *offsets, size_t n_msm,
                          uint8_t *outs, uint8_t *status);
